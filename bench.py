@@ -22,6 +22,10 @@ Full-size secondary configurations run behind --config:
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--skip-topk] [--skip-api]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` writes what the last timed step returned, as DIR/<name>.npy: the headline's embeddings and, unless
+--skip-topk, the merged top-k (doc, row, score).  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -320,7 +324,16 @@ def make_ctx(args):
         return float(t.item())
 
     c.barrier, c.max_over_ranks, c.sum_over_ranks = barrier, max_over_ranks, sum_over_ranks
+    c.outputs = {}                                  # name -> array returned by the last timed step (--dump-outputs)
     return c
+
+
+def dump_outputs(directory: str, outputs: dict):
+    """DIR/<name>.npy per array: float32 stays float32, any other dtype (ids, fp64 scores) is written as float64."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        np.save(os.path.join(directory, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 def timed_steps(c, step, steps: int, warmup: int):
@@ -385,6 +398,8 @@ def bench_headline(c):
     ev1.record(c.stream)
     c.barrier()
     w1 = time.perf_counter()
+    if args.dump_outputs:
+        c.outputs["embeddings"] = out_dev.cpu().numpy()
     launches = enc.last_timing()[1] * args.steps
     step_ms = c.max_over_ranks(ev0.elapsed_time(ev1)) / args.steps
     clocks = sampler.stop(w0, w1) if c.rank == 0 else None
@@ -494,6 +509,9 @@ def bench_topk(c):
     s1.record(stream)
     c.barrier()
     t_ms = c.max_over_ranks(s0.elapsed_time(s1)) / args.steps
+    if args.dump_outputs:
+        D, R, S = unpack_blocks(fin.cpu().numpy(), 1, TOPK_NQ, TOPK_K)
+        c.outputs.update(topk_doc=D[0], topk_row=R[0], topk_score=S[0])
     for _ in range(max(5, min(args.steps, 20))):   # per-kernel times (roofline numerator): CUDA events around the scan
         search_step()
         a, b = store.last_timing()
@@ -858,7 +876,13 @@ def main():
     ap.add_argument("--docs", type=int, default=100_000)
     ap.add_argument("--chunks", type=int, default=1_000_000)
     ap.add_argument("--pad-fraction", type=float, default=0.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (headline configuration only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "headline"):
+        ap.error("--dump-outputs covers the headline configuration of --impl b200 only")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.quick:
         args.skip_api = args.skip_cfg = True
@@ -909,6 +933,8 @@ def main():
             "gpu_launches": head["gpu_launches"], "clocks": head["clocks"], "cpu_baseline": cpu, "topk": topk,
             "api_e2e": api, "cfg2": cfg2, "cfg3": cfg3,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, c.outputs)
         emit(line)
     if c.distributed:
         dist.barrier()

@@ -17,6 +17,7 @@ Caveat recorded in the fixture: transformers here is 5.5.0 (reference pins 4.41.
 
 Run:  python tests/golden/make_reference_golden.py
 """
+import hashlib
 import json
 import os
 import sys
@@ -198,8 +199,9 @@ from PIL import Image  # noqa: E402
 
 imgs_sq = rng.integers(0, 256, size=(3, 224, 224, 3), dtype=np.uint8)
 imgs_big = rng.integers(0, 256, size=(2, 300, 400, 3), dtype=np.uint8)
-out["a3_images_224"] = imgs_sq
-out["a3_images_300x400"] = imgs_big
+# the test regenerates the pixels from this seeded stream (1.2 MB that does not compress); it checks these digests
+meta["a3_images_sha256"] = {"224": hashlib.sha256(imgs_sq.tobytes()).hexdigest(),
+                            "300x400": hashlib.sha256(imgs_big.tobytes()).hexdigest()}
 out["a3_vec_224"] = np.asarray(oc.encode_image([Image.fromarray(a) for a in imgs_sq], normalize=True), np.float32)
 out["a3_vec_300x400"] = np.asarray(oc.encode_image([Image.fromarray(a) for a in imgs_big], normalize=True), np.float32)
 out["a3_vec_224_unnormalized"] = np.asarray(oc.encode_image([Image.fromarray(a) for a in imgs_sq], normalize=False),

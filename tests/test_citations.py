@@ -1,32 +1,23 @@
-"""Every `file.py:line` citation of the reference in the header, the sources and the docs must name a file that exists
-under /root/reference with at least that many lines.  Runs only where the reference is mounted (the build container)."""
+"""Every `file.py:line` citation of the reference in the header, the sources and the docs must name a file of the
+reference project with at least that many lines.  The reference's files and line counts are recorded in
+tests/golden/reference_line_counts.json (tests/golden/make_citation_golden.py)."""
 import collections
 import glob
+import json
 import os
 import re
 
-import pytest
-
-REF = "/root/reference"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLD = os.path.join(ROOT, "tests", "golden", "reference_line_counts.json")
 PAT = re.compile(r"([A-Za-z0-9_./…-]*[A-Za-z0-9_]+\.(?:py|java|xml|sd))\s*:\s*(\d+(?:[-–]\d+)?(?:\s*,\s*:?\d+(?:[-–]\d+)?)*)")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted here")
 def test_reference_citations_resolve():
+    with open(GOLD) as fh:
+        lines = json.load(fh)
     by_name = collections.defaultdict(list)
-    for root, _, files in os.walk(REF):
-        if "/.git" in root:
-            continue
-        for f in files:
-            by_name[f].append(os.path.join(root, f))
-    lines = {}
-
-    def nlines(p):
-        if p not in lines:
-            with open(p, errors="ignore") as fh:
-                lines[p] = sum(1 for _ in fh)
-        return lines[p]
+    for p in lines:
+        by_name[os.path.basename(p)].append(p)
 
     sources = glob.glob(f"{ROOT}/include/*.h") + glob.glob(f"{ROOT}/marqo_b200/**/*.py", recursive=True) + \
         glob.glob(f"{ROOT}/marqo_b200/csrc/*.cu*") + glob.glob(f"{ROOT}/oracle/*.py") + glob.glob(f"{ROOT}/oracle/*.c") + \
@@ -47,6 +38,6 @@ def test_reference_citations_resolve():
             narrowed = [c for c in cands if c.endswith(path)] or cands
             top = max(int(x) for x in re.findall(r"\d+", m.group(2)))
             checked += 1
-            if not any(top <= nlines(c) for c in narrowed):
+            if not any(top <= lines[c] for c in narrowed):
                 bad.append((os.path.relpath(src, ROOT), m.group(0), f"line {top} past the end"))
     assert checked > 100 and not bad, bad[:20]
