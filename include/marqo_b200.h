@@ -381,9 +381,10 @@ int b200_jpeg_decode_batch(int device, const uint8_t* const* files, const size_t
 
 /* out[M,N] = act(A[M,K] @ W[N,K]^T + bias) (+ residual); A and W are rounded to bf16 on the device, fp32
  * accumulate; act: 0 none, 1 erf-GELU, 2 QuickGELU; bias/residual may be NULL; out_bf16 != 0 rounds the result to
- * bf16 before it is returned as fp32. */
+ * bf16 before it is returned as fp32.  in_place != 0 (needs a residual and fp32 output): the device output buffer IS
+ * the residual buffer, as in the model's out_proj / fc2, which add onto the residual stream they overwrite. */
 int b200_debug_gemm(int device, const float* A, const float* W, const float* bias, const float* residual, int M, int N,
-                    int K, int act, int out_bf16, float* out);
+                    int K, int act, int out_bf16, int in_place, float* out);
 /* Residual GEMM with the LayerNorm fused into its epilogue (gemm.cuh Epilogue::ln_*): out_x fp32 [M,N] = A W^T + bias
  * (+ residual); out_ln = LayerNorm(out_x) * gamma + beta rounded to bf16 (returned as fp32).  in_place != 0: the fp32
  * normalised rows also replace out_x (BERT post-LN).  The launch is repeated `repeats` times, alternating between two strip

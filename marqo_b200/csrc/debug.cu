@@ -164,20 +164,22 @@ int b200_debug_gemm_ln(int device, const float* A, const float* W, const float* 
 }
 
 int b200_debug_gemm(int device, const float* A, const float* W, const float* bias, const float* residual, int M, int N,
-                    int K, int act, int out_bf16, float* out) {
+                    int K, int act, int out_bf16, int in_place, float* out) {
     return guarded([&] {
         MB_CHECK_ARG(A && W && out, "NULL buffer");
         MB_CHECK_ARG(M > 0 && N > 0 && K > 0, "M, N, K must be positive");
+        MB_CHECK_ARG(!in_place || (residual && !out_bf16), "in_place needs a residual and fp32 output");
         require_device(device);
         DeviceGuard g(device);
         Scratch sc;
         MB_CUDA(cudaStreamCreate(&sc.s));
         __nv_bfloat16* dA = sc.upload_bf16(A, (size_t)M * K);
         __nv_bfloat16* dW = sc.upload_bf16(W, (size_t)N * K);
-        float* dOut = sc.alloc<float>((size_t)M * N);
+        // in place: the residual is uploaded into the output buffer, as out_proj / fc2 add onto the residual stream
+        float* dOut = in_place ? sc.upload(residual, (size_t)M * N) : sc.alloc<float>((size_t)M * N);
         gemm::Epilogue ep;
         ep.bias = bias ? sc.upload(bias, (size_t)N) : nullptr;
-        ep.residual = residual ? sc.upload(residual, (size_t)M * N) : nullptr;
+        ep.residual = in_place ? dOut : residual ? sc.upload(residual, (size_t)M * N) : nullptr;
         ep.ldr = N;
         ep.act = act;
         ep.ldo = N;

@@ -477,7 +477,10 @@ class Encoder:
 # ---------------------------------------------------------------------------------------------------------
 # Kernel-level diagnostics (b200_debug_*)
 # ---------------------------------------------------------------------------------------------------------
-def debug_gemm(A, W, bias=None, residual=None, act: int = 0, out_bf16: bool = False, device: int = 0) -> np.ndarray:
+def debug_gemm(A, W, bias=None, residual=None, act: int = 0, out_bf16: bool = False, in_place: bool = False,
+               device: int = 0) -> np.ndarray:
+    """act(A @ W^T + bias) (+ residual).  in_place: the kernel writes over the residual's device buffer, as out_proj
+    and fc2 write over the residual stream (needs a residual and fp32 output)."""
     A, W = _as(A, np.float32), _as(W, np.float32)
     M, K = A.shape
     Nn = W.shape[0]
@@ -485,7 +488,7 @@ def debug_gemm(A, W, bias=None, residual=None, act: int = 0, out_bf16: bool = Fa
     r = None if residual is None else _as(residual, np.float32)
     out = np.empty((M, Nn), np.float32)
     N.check(N.load().b200_debug_gemm(device, _ptr(A), _ptr(W), _ptr(b), _ptr(r), M, Nn, K, act, 1 if out_bf16 else 0,
-                                     _ptr(out)))
+                                     1 if in_place else 0, _ptr(out)))
     return out
 
 

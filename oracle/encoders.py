@@ -1,4 +1,6 @@
 """ORACLE — TEST INFRASTRUCTURE ONLY.  CPU fp32 restatement of the encoder arithmetic the reference calls into.
+The forwards take a `dtype` (default float32) and run on their input's device: the GPU tests run them in float64 on the
+GPU as a high-precision reference for every item of the production batches.
 
 The reference only *calls* third-party forwards (none of them vendored under /root/reference):
   * open_clip_torch==2.24.0 (requirements.dev.txt:33)  `model.encode_image` / `model.encode_text`, called at
@@ -208,12 +210,20 @@ def _l2_normalize_clip(out: torch.Tensor) -> torch.Tensor:
     return out / out.norm(dim=-1, keepdim=True)
 
 
+def _cast(sd, dtype: torch.dtype, device: torch.device):
+    """The weights in the compute type on the input's device (no copy when they already are)."""
+    return {k: v.to(device=device, dtype=dtype) for k, v in sd.items()}
+
+
 @torch.no_grad()
-def clip_encode_image(sd, cfg: ClipCfg, pixels: torch.Tensor, normalize: bool = True) -> torch.Tensor:
+def clip_encode_image(sd, cfg: ClipCfg, pixels: torch.Tensor, normalize: bool = True,
+                      dtype: torch.dtype = torch.float32) -> torch.Tensor:
     """pixels: fp32 [B,3,S,S] already preprocessed.  open_clip VisionTransformer forward (eval), then Marqo's cast +
-    L2 normalise."""
+    L2 normalise.  dtype: the compute type (float64 gives a high-precision reference; the output keeps it); the
+    weights are cast to it on the pixels' device."""
     v = cfg.vision
-    x = F.conv2d(pixels.float(), sd["visual.conv1.weight"], None, stride=v.patch)  # [B, W, g, g]
+    sd = _cast(sd, dtype, pixels.device)
+    x = F.conv2d(pixels.to(dtype), sd["visual.conv1.weight"], None, stride=v.patch)  # [B, W, g, g]
     B = x.shape[0]
     x = x.reshape(B, v.width, -1).permute(0, 2, 1)                                 # [B, g*g, W]
     cls = sd["visual.class_embedding"].expand(B, 1, v.width)
@@ -221,40 +231,45 @@ def clip_encode_image(sd, cfg: ClipCfg, pixels: torch.Tensor, normalize: bool = 
     x = F.layer_norm(x, (v.width,), sd["visual.ln_pre.weight"], sd["visual.ln_pre.bias"], 1e-5)
     x = _clip_tower(x, sd, "visual.", v, cfg.act, None)
     pooled = F.layer_norm(x[:, 0], (v.width,), sd["visual.ln_post.weight"], sd["visual.ln_post.bias"], 1e-5)
-    out = (pooled @ sd["visual.proj"]).to(torch.float32)
+    out = (pooled @ sd["visual.proj"]).to(dtype)
     return _l2_normalize_clip(out) if normalize else out
 
 
 @torch.no_grad()
-def clip_encode_text(sd, cfg: ClipCfg, ids: torch.Tensor, normalize: bool = True) -> torch.Tensor:
-    """ids: int [B, ctx].  open_clip text tower: causal mask, ln_final, EOT (= arg-max id) pooling, projection."""
+def clip_encode_text(sd, cfg: ClipCfg, ids: torch.Tensor, normalize: bool = True,
+                     dtype: torch.dtype = torch.float32) -> torch.Tensor:
+    """ids: int [B, ctx].  open_clip text tower: causal mask, ln_final, EOT (= arg-max id) pooling, projection.
+    dtype: the compute type, on the ids' device (as for clip_encode_image)."""
     t = cfg.text
     ids = ids.long()
     B, S = ids.shape
+    sd = _cast(sd, dtype, ids.device)
     x = sd["token_embedding.weight"][ids] + sd["positional_embedding"][:S]
-    mask = torch.full((S, S), float("-inf")).triu_(1)
+    mask = torch.full((S, S), float("-inf"), dtype=dtype, device=ids.device).triu_(1)
     x = _clip_tower(x, sd, "", t, cfg.act, mask)
     x = F.layer_norm(x, (t.width,), sd["ln_final.weight"], sd["ln_final.bias"], 1e-5)
-    pooled = x[torch.arange(B), ids.argmax(dim=-1)]
-    out = (pooled @ sd["text_projection"]).to(torch.float32)
+    pooled = x[torch.arange(B, device=ids.device), ids.argmax(dim=-1)]
+    out = (pooled @ sd["text_projection"]).to(dtype)
     return _l2_normalize_clip(out) if normalize else out
 
 
 @torch.no_grad()
 def bert_encode(sd, cfg: BertCfg, ids: torch.Tensor, attn_mask: Optional[torch.Tensor] = None,
-                normalize: bool = True) -> torch.Tensor:
+                normalize: bool = True, dtype: torch.dtype = torch.float32) -> torch.Tensor:
     """HF BertModel forward (post-LN, erf-GELU, additive key-padding mask) + Marqo's pooling / normalise
-    (hugging_face_model.py:188-214)."""
+    (hugging_face_model.py:188-214).  dtype: the compute type, on the ids' device; the mask fill is that type's
+    finfo.min, as BertModel's get_extended_attention_mask does for its own dtype."""
     ids = ids.long()
     B, S = ids.shape
+    sd = _cast(sd, dtype, ids.device)
     if attn_mask is None:
-        attn_mask = torch.ones(B, S, dtype=torch.long)
-    attn_mask = attn_mask.long()
+        attn_mask = torch.ones(B, S, dtype=torch.long, device=ids.device)
+    attn_mask = attn_mask.to(ids.device).long()
     w, hd = cfg.width, cfg.width // cfg.heads
     x = (sd["embeddings.word_embeddings.weight"][ids] + sd["embeddings.position_embeddings.weight"][:S]
          + sd["embeddings.token_type_embeddings.weight"][0])
     x = F.layer_norm(x, (w,), sd["embeddings.LayerNorm.weight"], sd["embeddings.LayerNorm.bias"], cfg.ln_eps)
-    add_mask = (1.0 - attn_mask[:, None, None, :].float()) * torch.finfo(torch.float32).min
+    add_mask = (1.0 - attn_mask[:, None, None, :].to(dtype)) * torch.finfo(dtype).min
     for i in range(cfg.layers):
         p = f"encoder.layer.{i}."
         q = F.linear(x, sd[p + "attention.self.query.weight"], sd[p + "attention.self.query.bias"])

@@ -119,3 +119,37 @@ def test_preprocess_identity_size_is_pure_normalise():
     ref = (torch.from_numpy(img).permute(0, 3, 1, 2).float() / 255.0
            - torch.tensor(E.OPENAI_CLIP_MEAN).view(1, 3, 1, 1)) / torch.tensor(E.OPENAI_CLIP_STD).view(1, 3, 1, 1)
     torch.testing.assert_close(got, ref, rtol=0, atol=1e-6)
+
+
+@pytest.mark.parametrize("arch", ["clip_gelu", "clip_quickgelu", "bert_mean", "bert_cls"])
+def test_oracle_dtype_argument(arch):
+    """The oracle's compute type is a parameter (float64 gives the high-precision reference of the GPU tests): the
+    tiny configurations agree across float32 / float64 to cosine 1 - 1e-6, and each output keeps its dtype."""
+    outs = {}
+    for dt in (torch.float32, torch.float64):
+        if arch.startswith("clip"):
+            cfg = E.tiny_clip(arch.split("_")[1])
+            sd = E.make_clip_weights(cfg, seed=5)
+            px = torch.randn(3, 3, 224, 224, generator=torch.Generator().manual_seed(1))
+            ids = torch.zeros(3, 77, dtype=torch.int64)
+            ids[:, 0] = cfg.text.vocab - 2
+            ids[:, 1:20] = torch.randint(1, cfg.text.vocab - 2, (3, 19), generator=torch.Generator().manual_seed(2))
+            ids[:, 20] = cfg.text.vocab - 1
+            ids[1, 3:] = 0
+            ids[1, 2] = cfg.text.vocab - 1
+            outs[dt] = [E.clip_encode_image(sd, cfg, px, dtype=dt), E.clip_encode_text(sd, cfg, ids, dtype=dt),
+                        E.clip_encode_image(sd, cfg, px, normalize=False, dtype=dt)]
+        else:
+            cfg = E.tiny_bert(arch.split("_")[1])
+            sd = E.make_bert_weights(cfg, seed=6)
+            ids = torch.randint(1, cfg.vocab, (4, 30), generator=torch.Generator().manual_seed(4))
+            mask = torch.ones(4, 30, dtype=torch.int64)
+            mask[1, 7:] = 0
+            mask[3, 1:] = 0
+            outs[dt] = [E.bert_encode(sd, cfg, ids, mask, dtype=dt), E.bert_encode(sd, cfg, ids, None, dtype=dt),
+                        E.bert_encode(sd, cfg, ids, mask, normalize=False, dtype=dt)]
+    for a, b in zip(outs[torch.float32], outs[torch.float64]):
+        assert a.dtype == torch.float32 and b.dtype == torch.float64
+        cos = torch.nn.functional.cosine_similarity(a.double(), b, dim=-1)
+        assert float((1 - cos).max()) < 1e-6, f"float32 vs float64 oracle: min cosine {float(cos.min())}"
+        torch.testing.assert_close(a.double().norm(dim=-1), b.norm(dim=-1), rtol=1e-5, atol=0)
