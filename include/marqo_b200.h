@@ -235,7 +235,11 @@ typedef struct b200_model b200_model;
 
 enum b200_arch {
     B200_ARCH_CLIP = 0, /* open_clip CLIP: vision tower + text tower */
-    B200_ARCH_BERT = 1  /* HF BertModel + pooling */
+    B200_ARCH_BERT = 1, /* HF BertModel + pooling */
+    B200_ARCH_MPNET = 2 /* HF MPNetModel + pooling (all-mpnet-base-v2 family): post-LN blocks as BERT with LayerNorm eps
+                           1e-5, a learned relative-position bias in every attention, no token-type embedding, position
+                           ids from 2 (padding index 1); text.ctx = max_position_embeddings (514), so sequences are at
+                           most ctx - 2 tokens; type_vocab is ignored */
 };
 enum b200_act { B200_ACT_GELU = 0, B200_ACT_QUICKGELU = 1 };
 enum b200_pool { B200_POOL_MEAN = 0, B200_POOL_CLS = 1 };
@@ -253,22 +257,23 @@ typedef struct b200_tower_desc {
 
 typedef struct b200_model_desc {
     int32_t arch;      /* enum b200_arch */
-    int32_t embed_dim; /* output dimension (CLIP projection dim; BERT: == width) */
+    int32_t embed_dim; /* output dimension (CLIP projection dim; BERT / MPNet: == width) */
     int32_t act;       /* enum b200_act */
-    int32_t pool;      /* BERT only: enum b200_pool (hugging_face_model.py:205-214) */
+    int32_t pool;      /* BERT / MPNet: enum b200_pool (hugging_face_model.py:205-214) */
     int32_t type_vocab; /* BERT only: token_type vocabulary (2) */
     int32_t max_batch; /* workspace sizing: largest number of items per encode call */
     float image_mean[3]; /* Normalize() constants, src/marqo/s2_inference/clip_utils.py:32-33 */
     float image_std[3];
     b200_tower_desc vision; /* CLIP only */
-    b200_tower_desc text;   /* CLIP text tower, or the BERT encoder */
+    b200_tower_desc text;   /* CLIP text tower, or the BERT / MPNet encoder */
 } b200_model_desc;
 
 int b200_model_create(int device, const b200_model_desc* desc, b200_model** out);
 int b200_model_destroy(b200_model* m);
 /* Upload one parameter (fp32, host, contiguous) under its checkpoint name: open_clip
  * state_dict names for CLIP ("visual.conv1.weight", "transformer.resblocks.0.attn.in_proj_weight",
- * ...), HF BertModel names for BERT ("embeddings.word_embeddings.weight", ...). */
+ * ...), HF BertModel names for BERT ("embeddings.word_embeddings.weight", ...), HF MPNetModel names for MPNet
+ * ("encoder.layer.0.attention.attn.q.weight", "encoder.relative_attention_bias.weight" [32, heads], ...). */
 int b200_model_load_tensor(b200_model* m, const char* name, const float* data, int64_t numel);
 /* Verifies every required parameter has been supplied, builds derived buffers. */
 int b200_model_finalize(b200_model* m);
@@ -286,7 +291,8 @@ int b200_model_encode_images_u8(b200_model* m, const uint8_t* hwc, int n, int h,
  * unchanged: abstract_clip_model.py:108-111). */
 int b200_model_encode_images_f32(b200_model* m, const float* chw, int n, int normalize, float* out);
 /* Token ids int32 [n, seq] (host).  CLIP: causal text tower, EOT = arg-max id pooling.
- * BERT: attn_mask int32 [n, seq] (1 = token, 0 = pad; NULL = all ones), token_type 0. */
+ * BERT: attn_mask int32 [n, seq] (1 = token, 0 = pad; NULL = all ones), token_type 0.
+ * MPNet: as BERT; token t of a row has position id 2 + t, pad tokens (mask 0) position id 1. */
 int b200_model_encode_tokens(b200_model* m, const int32_t* ids, const int32_t* attn_mask, int n, int seq,
                              int normalize, float* out);
 /* Device-resident variants: inputs/outputs are device pointers on the model's device,
@@ -322,6 +328,12 @@ typedef struct b200_tokenizer b200_tokenizer;
  * (one token per line, id = line number; must contain [PAD] [UNK] [CLS] [SEP]).  do_lower_case != 0 also strips
  * accents (BertNormalizer's strip_accents=None follows lowercase). */
 int b200_tokenizer_create_wordpiece(const char* vocab_utf8, size_t nbytes, int do_lower_case, b200_tokenizer** out);
+/* The same WordPiece with other special tokens: cls / sep frame every row, pad fills it, unk replaces unknown words;
+ * all four must be in the vocabulary.  MPNet's tokenizer is ("<s>", "</s>", "<pad>", "[UNK]").  Together with the four,
+ * the mask token is matched verbatim in the text when it is in the vocabulary: "[MASK]" when cls is "[CLS]", "<mask>"
+ * otherwise.  b200_tokenizer_create_wordpiece is this call with ("[CLS]", "[SEP]", "[PAD]", "[UNK]"). */
+int b200_tokenizer_create_wordpiece_special(const char* vocab_utf8, size_t nbytes, int do_lower_case, const char* cls,
+                                            const char* sep, const char* pad, const char* unk, b200_tokenizer** out);
 /* CLIP byte-level BPE — open_clip's SimpleTokenizer, the tokenizer OPEN_CLIP.load_tokenizer() returns for non-hf-hub
  * models (src/marqo/core/inference/embedding_models/open_clip_model.py:211-222; cleaning rules restated at
  * src/marqo/core/inference/embedding_models/hf_tokenizer.py:9-17).  merges_utf8: the DECOMPRESSED bytes of
@@ -402,6 +414,13 @@ int b200_debug_patch_embed(int device, const uint8_t* hwc, int n, int S, int pat
  * 2 key length (kv_len int32 [B]).  out fp32 [B*S, W]. */
 int b200_debug_attention(int device, const float* qkv, int B, int S, int W, int H, int mask, const int32_t* kv_len,
                          float* out);
+/* b200_debug_attention with MPNet's relative-position bias: score(i, j) += rel_bias[bucket(j - i)][h] (rel_bias fp32
+ * [32, H], host; bucket as transformers' MPNetEncoder.relative_position_bucket).  mask: 0 none or 2 key length. */
+int b200_debug_attention_relbias(int device, const float* qkv, int B, int S, int W, int H, int mask,
+                                 const int32_t* kv_len, const float* rel_bias, float* out);
+/* The library's relative-position buckets (host only, no device): out[d + max_distance] = bucket(d) for
+ * d = key - query in [-max_distance, max_distance]. */
+int b200_debug_relative_position_buckets(int max_distance, int32_t* out);
 /* LayerNorm over rows of fp32 [rows, w]. */
 /* Mean device time (ms, CUDA events) of `iters` back-to-back attention launches on device-generated data. */
 int b200_debug_attention_time(int device, int B, int S, int W, int H, int mask, int iters, float* out_ms);

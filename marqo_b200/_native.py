@@ -14,7 +14,7 @@ _lock = threading.Lock()
 OK, ERR_INVALID_ARG, ERR_NO_DEVICE, ERR_CUDA, ERR_OOM, ERR_UNSUPPORTED, ERR_INTERNAL, ERR_MISSING_WEIGHT = range(8)
 
 METRIC_PRENORMALIZED_ANGULAR, METRIC_ANGULAR, METRIC_DOTPRODUCT, METRIC_EUCLIDEAN = range(4)
-ARCH_CLIP, ARCH_BERT = 0, 1
+ARCH_CLIP, ARCH_BERT, ARCH_MPNET = 0, 1, 2
 ACT_GELU, ACT_QUICKGELU = 0, 1
 POOL_MEAN, POOL_CLS = 0, 1
 MAX_ATTRIBUTE_COLUMNS = 64
@@ -111,6 +111,8 @@ _SIGNATURES = {
     "b200_debug_gemm_ln": (C.c_int, [C.c_int, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P, C.c_float, C.c_int, C.c_int, _P, _P]),
     "b200_debug_patch_embed": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, C.c_int, _P]),
     "b200_debug_attention": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "b200_debug_attention_relbias": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
+    "b200_debug_relative_position_buckets": (C.c_int, [C.c_int, _P]),
     "b200_debug_attention_time": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float)]),
     "b200_debug_layernorm": (C.c_int, [C.c_int, _P, _P, _P, C.c_float, C.c_int, C.c_int, _P]),
     "b200_debug_resize": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
@@ -118,6 +120,8 @@ _SIGNATURES = {
     "b200_jpeg_decode_batch": (C.c_int, [C.c_int, _P, _P, C.c_int, _P, _P, _P, _P]),
     "b200_debug_jpeg_decode_host": (C.c_int, [_P, C.c_size_t, _P, C.c_size_t, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "b200_tokenizer_create_wordpiece": (C.c_int, [C.c_char_p, C.c_size_t, C.c_int, C.POINTER(_P)]),
+    "b200_tokenizer_create_wordpiece_special": (C.c_int, [C.c_char_p, C.c_size_t, C.c_int, C.c_char_p, C.c_char_p,
+                                                          C.c_char_p, C.c_char_p, C.POINTER(_P)]),
     "b200_tokenizer_create_clip_bpe": (C.c_int, [C.c_char_p, C.c_size_t, C.POINTER(_P)]),
     "b200_tokenizer_destroy": (C.c_int, [_P]),
     "b200_tokenizer_vocab_size": (C.c_int, [_P, C.POINTER(C.c_int)]),

@@ -16,6 +16,8 @@
 // against the 128 rows of the item and its V row are staged in smem for the epilogue; the row runs on mma.sync
 // against the K / V tiles while they sit in shared memory.
 // 113 KB smem + 256 TMEM columns per CTA -> two CTAs per SM, so one CTA's softmax overlaps the other's MMAs.
+// BIAS (MPNet): a learned relative-position bias per (head, key - query) enters every score before the softmax; warp 6
+// stages the item's head row of the bias in shared memory instead of handling a remainder key / row.
 #include <algorithm>
 #include <cstdlib>
 #include <mutex>
@@ -42,6 +44,11 @@ constexpr uint32_t TAILV_BYTES = HD * 2;                     // the remainder ke
 constexpr uint32_t SMEM_BYTES =
     Q_BYTES + KV_STAGES * 2 * KV_TILE_BYTES + P_BYTES + 128 + TAILS_BYTES + TAILV_BYTES;
 static_assert(SMEM_BYTES <= 115712, "two CTAs per SM");
+// BIAS: the staged head row of the relative-position bias (REL_T fp32) takes the place of the remainder key's scores
+// and V row: there is no room for both, so sequences of k * 128 + 1 tokens run their last key / query on a masked block
+constexpr uint32_t BIAS_ROW_BYTES = (REL_T * 4 + 15) / 16 * 16;
+constexpr uint32_t SMEM_BYTES_BIAS = Q_BYTES + KV_STAGES * 2 * KV_TILE_BYTES + P_BYTES + 128 + BIAS_ROW_BYTES;
+static_assert(SMEM_BYTES_BIAS <= 115712, "two CTAs per SM");
 constexpr uint32_t TMEM_COLS = 256;
 constexpr uint32_t S_COL = 0, O_COL = 128;
 constexpr int DEFAULT_SOFTMAX_MODE = 1;
@@ -91,19 +98,33 @@ __device__ __forceinline__ void tmem_ld_wait_regs16(uint32_t (&v)[16]) {
                  : "memory");
 }
 
+// Relative-position bias of key - query = d (log2 units): sB points at the staged head row's d = 0 entry.
+__device__ __forceinline__ float rel_bias(const float* sB, int d) { return sB[min(max(d, -REL_D), REL_D)]; }
+
 // 16 keys (block-local columns k0 .. k0 + 15) of a score row with FOUR independent sum / max chains: the softmax warps
 // are latency-bound (two of them per scheduler), so the serial `lsum += p` chain of the 32-key version below costs
 // more than its instructions.
-template <bool FULL>
+// BIAS: the scores are x = s * scale_log2e + bias (dk = block key 0 - query) and mx tracks x, not the raw s.
+template <bool FULL, bool BIAS = false>
 __device__ __forceinline__ void softmax_half_chunk(const uint32_t (&v)[16], int k0, int klo, int khi, float scale_log2e,
-                                                   float m_safe, float (&ls)[4], float (&mx)[4], uint8_t* sP, int r) {
+                                                   float m_safe, float (&ls)[4], float (&mx)[4], uint8_t* sP, int r,
+                                                   const float* sB = nullptr, int dk = 0) {
     uint32_t pk[8];
 #pragma unroll
     for (int i = 0; i < 16; i += 2) {
         const float s0 = __uint_as_float(v[i]), s1 = __uint_as_float(v[i + 1]);
         float p0, p1;
         const int a = (i >> 1) & 3;
-        if (FULL) {
+        if constexpr (BIAS) {
+            const int kk = k0 + i;
+            const float x0 = fmaf(s0, scale_log2e, rel_bias(sB, dk + kk));
+            const float x1 = fmaf(s1, scale_log2e, rel_bias(sB, dk + kk + 1));
+            const bool ok0 = FULL || (kk >= klo && kk < khi), ok1 = FULL || (kk + 1 >= klo && kk + 1 < khi);
+            mx[a] = ok0 ? fmaxf(mx[a], x0) : mx[a];
+            mx[a] = ok1 ? fmaxf(mx[a], x1) : mx[a];
+            p0 = ok0 ? ex2(x0 - m_safe) : 0.f;
+            p1 = ok1 ? ex2(x1 - m_safe) : 0.f;
+        } else if (FULL) {
             mx[a] = fmaxf(mx[a], fmaxf(s0, s1));
             p0 = ex2(fmaf(s0, scale_log2e, -m_safe));
             p1 = ex2(fmaf(s1, scale_log2e, -m_safe));
@@ -127,15 +148,26 @@ __device__ __forceinline__ void softmax_half_chunk(const uint32_t (&v)[16], int 
 
 // One 32-key chunk of a score row: p = exp2(s * scale - m_safe) for the keys in [klo, khi) (block-local indices), 0 for
 // the others; running raw maximum, row sum, bf16 P into the K-major 128B-swizzled A-operand layout.
-template <bool FULL>
+// BIAS: as softmax_half_chunk.
+template <bool FULL, bool BIAS = false>
 __device__ __forceinline__ void softmax_chunk(const uint32_t (&v)[32], int c, int klo, int khi, float scale_log2e,
-                                              float m_safe, float& lsum, float& mx, uint8_t* sP, int r) {
+                                              float m_safe, float& lsum, float& mx, uint8_t* sP, int r,
+                                              const float* sB = nullptr, int dk = 0) {
     uint32_t pk[16];
 #pragma unroll
     for (int i = 0; i < 32; i += 2) {
         const float s0 = __uint_as_float(v[i]), s1 = __uint_as_float(v[i + 1]);
         float p0, p1;
-        if (FULL) {
+        if constexpr (BIAS) {
+            const int k0 = c * 32 + i;
+            const float x0 = fmaf(s0, scale_log2e, rel_bias(sB, dk + k0));
+            const float x1 = fmaf(s1, scale_log2e, rel_bias(sB, dk + k0 + 1));
+            const bool ok0 = FULL || (k0 >= klo && k0 < khi), ok1 = FULL || (k0 + 1 >= klo && k0 + 1 < khi);
+            mx = ok0 ? fmaxf(mx, x0) : mx;
+            mx = ok1 ? fmaxf(mx, x1) : mx;
+            p0 = ok0 ? ex2(x0 - m_safe) : 0.f;
+            p1 = ok1 ? ex2(x1 - m_safe) : 0.f;
+        } else if (FULL) {
             mx = fmaxf(mx, fmaxf(s0, s1));
             p0 = ex2(fmaf(s0, scale_log2e, -m_safe));
             p1 = ex2(fmaf(s1, scale_log2e, -m_safe));
@@ -199,11 +231,15 @@ __device__ __forceinline__ void item_extent(const Item& w, int S, int s_main, co
 // dropped to ONE CTA per SM and ran 1.85x slower.
 // SM: softmax schedule of the row threads — 0 two passes over S (exact block maximum), 1 one pass / one register buffer,
 // 2 one pass with the next chunk's tcgen05.ld in flight (two buffers).  All three use the lazy exponent reference.
-template <int MASK, bool PACKED, int SM>
+// BIAS: every score gets the relative-position bias of its head and of key - query (positions within the sequence, also
+// in packed tiles) before the softmax; warp 6 stages the item's head row of bias_log2 [H, REL_T] in shared memory
+// instead of handling a remainder key / row (the launcher never passes one).
+template <int MASK, bool PACKED, int SM, bool BIAS>
 __global__ void __launch_bounds__(THREADS, 2)
 attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat16* __restrict__ qkv,
                     __nv_bfloat16* __restrict__ out, int S, int W, int H, const int32_t* __restrict__ kv_len,
-                    float scale_log2e, int s_main, int inline_tail_rows, int q_blocks, int total_items, int pack, int B) {
+                    float scale_log2e, int s_main, int inline_tail_rows, int q_blocks, int total_items, int pack, int B,
+                    const float* __restrict__ bias_log2) {
     const int stride = PACKED ? pack * S : S;   // rows between the bases of consecutive sequences / groups
     // Keys [0, s_main) go through the tensor cores in blocks of 128; the few keys [s_main, S) of a sequence length
     // such as 257 = 2 * 128 + 1 (ViT class token) are folded in on the CUDA cores in the epilogue instead of paying
@@ -222,10 +258,11 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
     uint64_t* pv_done = bars + 8;
     uint64_t* q_empty = bars + 9;
     uint64_t* tail_full = bars + 10;    // the remainder key's scores + V row are staged (warp 6 -> softmax warps)
-    uint64_t* tail_empty = bars + 11;   // ... and have been consumed
+    uint64_t* tail_empty = bars + 11;   // ... and have been consumed (BIAS: the same for the bias row)
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 12);
     float* sTailS = reinterpret_cast<float*>(sP + P_BYTES + 128);
     __nv_bfloat16* sTailV = reinterpret_cast<__nv_bfloat16*>(sP + P_BYTES + 128 + TAILS_BYTES);
+    float* sBias = reinterpret_cast<float*>(sP + P_BYTES + 128);   // BIAS only: bias_log2[h][0 .. REL_T)
 
     const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
     const int lane = threadIdx.x & 31;
@@ -234,12 +271,13 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
     if (warp == 0 && lane == 0) {
         ptx::prefetch_tmap(&tmap);
         ptx::mbar_init(q_full, 1);
-        ptx::mbar_init(q_empty, 2);   // the MMA warp's commit after the item's last S + warp 6 (remainder-key scores)
+        // the MMA warp's commit after the item's last S + warp 6 (remainder-key scores; BIAS: warp 6 reads no tile)
+        ptx::mbar_init(q_empty, BIAS ? 1 : 2);
         ptx::mbar_init(tail_full, 1);
         ptx::mbar_init(tail_empty, 4);
         for (int i = 0; i < KV_STAGES; ++i) {
             ptx::mbar_init(&kv_full[i], 1);
-            ptx::mbar_init(&kv_empty[i], 2);   // the MMA warp's commit + the remainder-row warp
+            ptx::mbar_init(&kv_empty[i], BIAS ? 1 : 2);   // the MMA warp's commit + the remainder-row warp
         }
         ptx::mbar_init(s_full, 1);
         ptx::mbar_init(s_free, 4);
@@ -369,6 +407,24 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
             ++gp;
             advance(cp, false);
             if (!s_first && cs.it < total_items) issue_s();
+        }
+    } else if (warp == 6 && BIAS) {
+        // ================================================================== relative-bias row of each item's head
+        // loaded into registers before waiting for the softmax warps to release the previous row, so the L2 latency
+        // is hidden behind the previous item
+        uint32_t n = 0;
+        for (int it = blockIdx.x; it < total_items; it += gridDim.x, ++n) {
+            const Item w = decode_item(it, q_blocks, H);
+            const float* src = bias_log2 + (size_t)w.h * REL_T;
+            float v[(REL_T + 31) / 32];
+#pragma unroll
+            for (int u = 0; u < (REL_T + 31) / 32; ++u) v[u] = lane + 32 * u < REL_T ? __ldg(src + lane + 32 * u) : 0.f;
+            if (n > 0) ptx::mbar_wait(tail_empty, (n - 1) & 1);
+#pragma unroll
+            for (int u = 0; u < (REL_T + 31) / 32; ++u)
+                if (lane + 32 * u < REL_T) sBias[lane + 32 * u] = v[u];
+            __syncwarp();
+            if (lane == 0) ptx::mbar_arrive(tail_full);
         }
     } else if (warp == 6) {
         // ================================================================== remainder key + remainder query row
@@ -601,7 +657,12 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
             float m_run = -INFINITY, l_run = 0.f;
             // The remainder key (257 = 2 * 128 + 1) is folded in on the CUDA cores in the epilogue from the scores and
             // the V row that warp 6 stages in shared memory.
-            const bool has_tail_key = s_main < len;   // uniform over the CTA
+            const bool has_tail_key = !BIAS && s_main < len;   // uniform over the CTA
+            const float* sB = nullptr;   // BIAS: the staged row at distance 0
+            if constexpr (BIAS) {
+                ptx::mbar_wait(tail_full, nt & 1);
+                sB = sBias + REL_D;
+            }
             const int tail_end = qrow < S ? (MASK == MASK_CAUSAL ? min(len, qrow + 1) : len) : 0;
             for (int j = 0; j < nkb; ++j, ++g) {
                 const uint32_t par = g & 1;
@@ -615,6 +676,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                     khi = p_hi;
                 }
                 const bool full = klo <= 0 && khi >= BKV;
+                const int dk = j * BKV - qrow;   // BIAS: key - query of block-local key 0 (PACKED: tile rows = positions)
                 // The exponent reference of a row is LAZY: it only moves when the block's true maximum exceeds it by
                 // more than 2^8 (exp2(s - ref) <= 256 keeps P inside bf16's useful range and every sum far inside
                 // fp32), so after a row's first block the O accumulator is almost never rescaled.  All decisions are
@@ -627,7 +689,13 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                     for (int c = 0; c < BKV / 32; ++c) {
                         ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
                         tmem_ld_wait_regs(va);
-                        if (full) {
+                        if constexpr (BIAS) {
+#pragma unroll
+                            for (int i = 0; i < 32; ++i)
+                                if (full || (c * 32 + i >= klo && c * 32 + i < khi))
+                                    mx = fmaxf(mx, fmaf(__uint_as_float(va[i]), scale_log2e,
+                                                        rel_bias(sB, dk + c * 32 + i)));
+                        } else if (full) {
 #pragma unroll
                             for (int i = 0; i < 32; ++i) mx = fmaxf(mx, __uint_as_float(va[i]));
                         } else {
@@ -636,7 +704,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                                 if (c * 32 + i >= klo && c * 32 + i < khi) mx = fmaxf(mx, __uint_as_float(va[i]));
                         }
                     }
-                    const float bmax = mx * scale_log2e;   // scale > 0: max commutes with the scaling
+                    const float bmax = BIAS ? mx : mx * scale_log2e;   // scale > 0: max commutes with the scaling
                     const bool move = j == 0 || bmax > m_run + 8.0f;
                     if (move) m_new = fmaxf(m_run, bmax);
                     const float m_safe = m_new == -INFINITY ? 0.f : m_new;
@@ -647,8 +715,8 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                     for (int c = 0; c < BKV / 32; ++c) {
                         ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
                         tmem_ld_wait_regs(va);
-                        if (full) softmax_chunk<true>(va, c, klo, khi, scale_log2e, m_safe, lsum, dummy, sP, r);
-                        else softmax_chunk<false>(va, c, klo, khi, scale_log2e, m_safe, lsum, dummy, sP, r);
+                        if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, dummy, sP, r, sB, dk);
+                        else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, dummy, sP, r, sB, dk);
                     }
                 } else {
                     // ---- one pass: reference = running reference (first block: max of the row's first 32 scores);
@@ -658,10 +726,18 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                     float m_ref = m_run;
                     if (j == 0) {
                         float c0 = -INFINITY;
+                        if constexpr (BIAS) {
 #pragma unroll
-                        for (int i = 0; i < 32; ++i)
-                            if (full || (i >= klo && i < khi)) c0 = fmaxf(c0, __uint_as_float(va[i]));
-                        m_ref = c0 * scale_log2e;
+                            for (int i = 0; i < 32; ++i)
+                                if (full || (i >= klo && i < khi))
+                                    c0 = fmaxf(c0, fmaf(__uint_as_float(va[i]), scale_log2e, rel_bias(sB, dk + i)));
+                            m_ref = c0;
+                        } else {
+#pragma unroll
+                            for (int i = 0; i < 32; ++i)
+                                if (full || (i >= klo && i < khi)) c0 = fmaxf(c0, __uint_as_float(va[i]));
+                            m_ref = c0 * scale_log2e;
+                        }
                     }
                     const float m_safe = m_ref == -INFINITY ? 0.f : m_ref;
                     if (j > 0) ptx::mbar_wait(pv_done, par ^ 1);
@@ -678,12 +754,20 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                         for (int c = 0; c < BKV / 32; ++c) {
                             if (c > 0) tmem_ld_wait_regs16(vlo);
                             ptx::tmem_ld_32x32b_x16(lane_addr + S_COL + c * 32 + 16, vb);
-                            if (full) softmax_half_chunk<true>(vlo, c * 32, klo, khi, scale_log2e, m_safe, ls4, mx4, sP, r);
-                            else softmax_half_chunk<false>(vlo, c * 32, klo, khi, scale_log2e, m_safe, ls4, mx4, sP, r);
+                            if (full)
+                                softmax_half_chunk<true, BIAS>(vlo, c * 32, klo, khi, scale_log2e, m_safe, ls4, mx4, sP, r,
+                                                               sB, dk);
+                            else
+                                softmax_half_chunk<false, BIAS>(vlo, c * 32, klo, khi, scale_log2e, m_safe, ls4, mx4, sP,
+                                                                r, sB, dk);
                             tmem_ld_wait_regs16(vb);
                             if (c + 1 < BKV / 32) ptx::tmem_ld_32x32b_x16(lane_addr + S_COL + (c + 1) * 32, vlo);
-                            if (full) softmax_half_chunk<true>(vb, c * 32 + 16, klo, khi, scale_log2e, m_safe, ls4, mx4, sP, r);
-                            else softmax_half_chunk<false>(vb, c * 32 + 16, klo, khi, scale_log2e, m_safe, ls4, mx4, sP, r);
+                            if (full)
+                                softmax_half_chunk<true, BIAS>(vb, c * 32 + 16, klo, khi, scale_log2e, m_safe, ls4, mx4,
+                                                               sP, r, sB, dk);
+                            else
+                                softmax_half_chunk<false, BIAS>(vb, c * 32 + 16, klo, khi, scale_log2e, m_safe, ls4, mx4,
+                                                                sP, r, sB, dk);
                         }
                         lsum = (ls4[0] + ls4[1]) + (ls4[2] + ls4[3]);
                         mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
@@ -694,12 +778,12 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                                 ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
                                 tmem_ld_wait_regs(va);
                             }
-                            if (full) softmax_chunk<true>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r);
-                            else softmax_chunk<false>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r);
+                            if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r, sB, dk);
+                            else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r, sB, dk);
                         }
                     }
                     m_new = m_ref;
-                    const float m_true = fmaxf(m_ref, mx * scale_log2e);
+                    const float m_true = fmaxf(m_ref, BIAS ? mx : mx * scale_log2e);
                     const bool exceeded = m_true > m_safe + 8.0f;
                     if (__any_sync(0xffffffffu, exceeded)) {
                         // exact update for this block: reference = true running maximum, P recomputed
@@ -712,8 +796,8 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                         for (int c = 0; c < BKV / 32; ++c) {
                             ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
                             tmem_ld_wait_regs(va);
-                            if (full) softmax_chunk<true>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r);
-                            else softmax_chunk<false>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r);
+                            if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r, sB, dk);
+                            else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r, sB, dk);
                         }
                     }
                 }
@@ -740,6 +824,11 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                 ptx::tc_fence_before();
                 __syncwarp();
                 if (lane == 0) ptx::mbar_arrive(p_full);
+            }
+            if constexpr (BIAS) {   // the scores of this item are done: warp 6 may stage the next item's row
+                __syncwarp();
+                if (lane == 0) ptx::mbar_arrive(tail_empty);
+                ++nt;
             }
             // -------------------------------------------------------------- epilogue: (+ tail keys) O / l -> bf16
             // remainder key: online-softmax update of (m, l); the output is finished 32 dims at a time below
@@ -825,19 +914,35 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
 }  // namespace tc
 
 using KernelFn = void (*)(const CUtensorMap, const __nv_bfloat16*, __nv_bfloat16*, int, int, int, const int32_t*, float,
-                          int, int, int, int, int, int);
+                          int, int, int, int, int, int, const float*);
 
 template <int SM>
 static KernelFn kernel_for(int mask, bool packed) {
     static const KernelFn table[2][3] = {
-        {tc::attention_tc_kernel<MASK_NONE, false, SM>, tc::attention_tc_kernel<MASK_CAUSAL, false, SM>,
-         tc::attention_tc_kernel<MASK_KEYLEN, false, SM>},
-        {tc::attention_tc_kernel<MASK_NONE, true, SM>, tc::attention_tc_kernel<MASK_CAUSAL, true, SM>,
-         tc::attention_tc_kernel<MASK_KEYLEN, true, SM>}};
+        {tc::attention_tc_kernel<MASK_NONE, false, SM, false>, tc::attention_tc_kernel<MASK_CAUSAL, false, SM, false>,
+         tc::attention_tc_kernel<MASK_KEYLEN, false, SM, false>},
+        {tc::attention_tc_kernel<MASK_NONE, true, SM, false>, tc::attention_tc_kernel<MASK_CAUSAL, true, SM, false>,
+         tc::attention_tc_kernel<MASK_KEYLEN, true, SM, false>}};
     return table[packed ? 1 : 0][mask];
 }
 
-static KernelFn pick_kernel(int sm, int mask, bool packed) {
+// relative-position bias variants: MASK_NONE and MASK_KEYLEN (no model combines the bias with causal masking)
+template <int SM>
+static KernelFn bias_kernel_for(int mask, bool packed) {
+    static const KernelFn table[2][2] = {
+        {tc::attention_tc_kernel<MASK_NONE, false, SM, true>, tc::attention_tc_kernel<MASK_KEYLEN, false, SM, true>},
+        {tc::attention_tc_kernel<MASK_NONE, true, SM, true>, tc::attention_tc_kernel<MASK_KEYLEN, true, SM, true>}};
+    return table[packed ? 1 : 0][mask == MASK_KEYLEN ? 1 : 0];
+}
+
+static KernelFn pick_kernel(int sm, int mask, bool packed, bool bias = false) {
+    if (bias) {
+        switch (sm) {
+            case 0: return bias_kernel_for<0>(mask, packed);
+            case 2: return bias_kernel_for<2>(mask, packed);
+            default: return bias_kernel_for<1>(mask, packed);
+        }
+    }
     switch (sm) {
         case 0: return kernel_for<0>(mask, packed);
         case 2: return kernel_for<2>(mask, packed);
@@ -846,11 +951,15 @@ static KernelFn pick_kernel(int sm, int mask, bool packed) {
 }
 
 int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W, int H, int mask, const int32_t* kv_len,
-              cudaStream_t stream) {
+              const float* bias_log2, cudaStream_t stream) {
     if (B <= 0 || S <= 0) return 0;
     if (W != H * tc::HD) fail(B200_ERR_UNSUPPORTED, "attention: head_dim must be 64 (width %d, heads %d)", W, H);
     if (mask < MASK_NONE || mask > MASK_KEYLEN) fail(B200_ERR_INTERNAL, "attention: unknown mask mode %d", mask);
     if (mask == MASK_KEYLEN && !kv_len) fail(B200_ERR_INTERNAL, "attention: kv_len required for key-length masking");
+    const bool bias = bias_log2 != nullptr;
+    if (bias && mask == MASK_CAUSAL)
+        fail(B200_ERR_INTERNAL, "attention: causal masking takes no relative-position bias");
+    const uint32_t smem = bias ? tc::SMEM_BYTES_BIAS : tc::SMEM_BYTES;
     // softmax schedule (see the kernel's SM parameter); MARQO_B200_ATTN_SOFTMAX=0|1|2 overrides for A/B timing
     static const int softmax_mode = [] {
         const char* e = getenv("MARQO_B200_ATTN_SOFTMAX");
@@ -864,6 +973,16 @@ int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W,
                     MB_CUDA(cudaFuncSetAttribute(pick_kernel(sm, mk, pk != 0), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                  (int)tc::SMEM_BYTES));
     });
+    static std::once_flag once_bias;
+    if (bias)
+        std::call_once(once_bias, [] {
+            for (int sm = 0; sm < 3; ++sm)
+                for (int pk = 0; pk < 2; ++pk)
+                    for (int mk : {(int)MASK_NONE, (int)MASK_KEYLEN})
+                        MB_CUDA(cudaFuncSetAttribute(pick_kernel(sm, mk, pk != 0, true),
+                                                     cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                     (int)tc::SMEM_BYTES_BIAS));
+        });
     // one tensor map over the packed [B*S, 3W] matrix serves Q, K and V tiles (64 columns x 128 rows, 128B swizzle);
     // rows past the end of the matrix are zero-filled, rows of the next sequence are masked by key index
     CUtensorMap tmap = make_tmap_2d(qkv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)3 * W, (uint64_t)B * S,
@@ -878,15 +997,17 @@ int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W,
         const int groups = (B + pack - 1) / pack;
         const int total_items = groups * H;
         const int grid = std::min(2 * sm_count(device), total_items);
-        pick_kernel(softmax_mode, mask, true)<<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(
-            tmap, qkv, out, S, W, H, kv_len, scale_log2e, /*s_main=*/1 << 30, 0, /*q_blocks=*/1, total_items, pack, B);
+        pick_kernel(softmax_mode, mask, true, bias)<<<grid, tc::THREADS, smem, stream>>>(
+            tmap, qkv, out, S, W, H, kv_len, scale_log2e, /*s_main=*/1 << 30, 0, /*q_blocks=*/1, total_items, pack, B,
+            bias_log2);
         MB_CUDA(cudaGetLastError());
         return 1;
     }
     // A remainder of ONE token (S = 257, 129, ...: a class token on top of a power-of-two grid) is not worth a 128-wide
-    // tile in either dimension: warp 6 of the kernel handles that key and that query row.
+    // tile in either dimension: warp 6 of the kernel handles that key and that query row.  The bias variants use warp 6
+    // and the remainder's shared memory for the bias row instead and run such a sequence as one more masked block.
     const int rem = S % tc::BQ;
-    const bool tail = S > tc::BQ && rem == 1;
+    const bool tail = !bias && S > tc::BQ && rem == 1;
     const int s_main = tail ? S - rem : S;                       // keys handled by the tensor cores
     const int q_blocks = tail ? S / tc::BQ : (S + tc::BQ - 1) / tc::BQ;
     const int inline_rows = tail ? rem : 0;
@@ -896,8 +1017,8 @@ int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W,
     int grid = 2 * sm_count(device);
     if ((q_blocks & 1) == 0 && (grid & 1) == 0) grid -= 1;
     grid = std::min(grid, total_items);
-    pick_kernel(softmax_mode, mask, false)<<<grid, tc::THREADS, tc::SMEM_BYTES, stream>>>(
-        tmap, qkv, out, S, W, H, kv_len, scale_log2e, s_main, inline_rows, q_blocks, total_items, 1, B);
+    pick_kernel(softmax_mode, mask, false, bias)<<<grid, tc::THREADS, smem, stream>>>(
+        tmap, qkv, out, S, W, H, kv_len, scale_log2e, s_main, inline_rows, q_blocks, total_items, 1, B, bias_log2);
     MB_CUDA(cudaGetLastError());
     return 1;
 }

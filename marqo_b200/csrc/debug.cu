@@ -217,12 +217,47 @@ int b200_debug_attention(int device, const float* qkv, int B, int S, int W, int 
         __nv_bfloat16* dO = sc.alloc<__nv_bfloat16>(M * W);
         float* dOut = sc.alloc<float>(M * W);
         const int32_t* dlen = kv_len ? sc.upload(kv_len, (size_t)B) : nullptr;
-        attention::launch(dq, dO, B, S, W, H, mask, dlen, sc.s);
+        attention::launch(dq, dO, B, S, W, H, mask, dlen, nullptr, sc.s);
         const long long n = (long long)M * W;
         bf16_to_f32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, sc.s>>>(dO, dOut, n);
         MB_CUDA(cudaGetLastError());
         MB_CUDA(cudaStreamSynchronize(sc.s));
         MB_CUDA(cudaMemcpy(out, dOut, M * W * 4, cudaMemcpyDeviceToHost));
+    });
+}
+
+int b200_debug_attention_relbias(int device, const float* qkv, int B, int S, int W, int H, int mask,
+                                 const int32_t* kv_len, const float* rel_bias, float* out) {
+    return guarded([&] {
+        MB_CHECK_ARG(qkv && rel_bias && out, "NULL buffer");
+        MB_CHECK_ARG(B > 0 && S > 0 && W > 0 && H > 0, "B, S, W, H must be positive");
+        MB_CHECK_ARG(mask == attention::MASK_NONE || mask == attention::MASK_KEYLEN, "mask must be 0 (none) or 2 (key length)");
+        require_device(device);
+        DeviceGuard g(device);
+        Scratch sc;
+        MB_CUDA(cudaStreamCreate(&sc.s));
+        const size_t M = (size_t)B * S;
+        std::vector<float> folded((size_t)H * attention::REL_T);
+        attention::fold_relative_bias(rel_bias, H, S - 1, folded.data());
+        const float* dbias = sc.upload(folded.data(), folded.size());
+        __nv_bfloat16* dq = sc.upload_bf16(qkv, M * 3 * W);
+        __nv_bfloat16* dO = sc.alloc<__nv_bfloat16>(M * W);
+        float* dOut = sc.alloc<float>(M * W);
+        const int32_t* dlen = kv_len ? sc.upload(kv_len, (size_t)B) : nullptr;
+        attention::launch(dq, dO, B, S, W, H, mask, dlen, dbias, sc.s);
+        const long long n = (long long)M * W;
+        bf16_to_f32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, sc.s>>>(dO, dOut, n);
+        MB_CUDA(cudaGetLastError());
+        MB_CUDA(cudaStreamSynchronize(sc.s));
+        MB_CUDA(cudaMemcpy(out, dOut, M * W * 4, cudaMemcpyDeviceToHost));
+    });
+}
+
+int b200_debug_relative_position_buckets(int max_distance, int32_t* out) {
+    return guarded([&] {
+        MB_CHECK_ARG(out != nullptr, "NULL buffer");
+        MB_CHECK_ARG(max_distance >= 0, "max_distance must be >= 0");
+        for (int d = -max_distance; d <= max_distance; ++d) out[d + max_distance] = attention::relative_position_bucket(d);
     });
 }
 
@@ -245,9 +280,9 @@ int b200_debug_attention_time(int device, int B, int S, int W, int H, int mask, 
         cudaEvent_t e0, e1;
         MB_CUDA(cudaEventCreate(&e0));
         MB_CUDA(cudaEventCreate(&e1));
-        for (int i = 0; i < 3; ++i) attention::launch(dq, dO, B, S, W, H, mask, dlen, sc.s);   // warm-up
+        for (int i = 0; i < 3; ++i) attention::launch(dq, dO, B, S, W, H, mask, dlen, nullptr, sc.s);   // warm-up
         MB_CUDA(cudaEventRecord(e0, sc.s));
-        for (int i = 0; i < iters; ++i) attention::launch(dq, dO, B, S, W, H, mask, dlen, sc.s);
+        for (int i = 0; i < iters; ++i) attention::launch(dq, dO, B, S, W, H, mask, dlen, nullptr, sc.s);
         MB_CUDA(cudaEventRecord(e1, sc.s));
         MB_CUDA(cudaStreamSynchronize(sc.s));
         float ms = 0.f;

@@ -205,6 +205,9 @@ void clip_text_embed(const int32_t* ids, const float* tok, const float* pos, int
     MB_CUDA(cudaGetLastError());
 }
 
+// MPNET: no token-type row, and the position id of token s is 2 + s (1, the padding index, for pad tokens): HF's
+// create_position_ids_from_input_ids on the right-padded rows the tokenizer produces
+template <bool MPNET>
 __global__ void __launch_bounds__(256) bert_embed_ln_kernel(const int32_t* __restrict__ ids, const int32_t* __restrict__ mask,
                                                             const float* __restrict__ word, const float* __restrict__ pos,
                                                             const float* __restrict__ type0, const float* __restrict__ gamma,
@@ -219,16 +222,22 @@ __global__ void __launch_bounds__(256) bert_embed_ln_kernel(const int32_t* __res
     id = min(max(id, 0), vocab - 1);
     const int nv = w / 128;
     const float4* w4 = reinterpret_cast<const float4*>(word + (long long)id * w);
-    const float4* p4 = reinterpret_cast<const float4*>(pos + (long long)s * w);
+    const int p = MPNET ? ((mask == nullptr || mask[row] != 0) ? 2 + s : 1) : s;
+    const float4* p4 = reinterpret_cast<const float4*>(pos + (long long)p * w);
     const float4* t4 = reinterpret_cast<const float4*>(type0);
     float4 v[LN_MAX_V4];
 #pragma unroll
     for (int j = 0; j < LN_MAX_V4; ++j)
         if (j < nv) {
             const int i4 = lane + 32 * j;
-            const float4 a = __ldg(w4 + i4), b = __ldg(p4 + i4), c = __ldg(t4 + i4);
-            // HF: inputs_embeds + token_type_embeddings, then + position_embeddings
-            v[j] = make_float4((a.x + c.x) + b.x, (a.y + c.y) + b.y, (a.z + c.z) + b.z, (a.w + c.w) + b.w);
+            if constexpr (MPNET) {   // HF: inputs_embeds + position_embeddings
+                const float4 a = __ldg(w4 + i4), b = __ldg(p4 + i4);
+                v[j] = make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
+            } else {
+                const float4 a = __ldg(w4 + i4), b = __ldg(p4 + i4), c = __ldg(t4 + i4);
+                // HF: inputs_embeds + token_type_embeddings, then + position_embeddings
+                v[j] = make_float4((a.x + c.x) + b.x, (a.y + c.y) + b.y, (a.z + c.z) + b.z, (a.w + c.w) + b.w);
+            }
         }
     ln_row<true>(v, nv, w, gamma, beta, eps, lane, x + row * w, h + row * w);
     if (s == 0 && lane == 0) {
@@ -247,8 +256,19 @@ void bert_embed_ln(const int32_t* ids, const int32_t* mask, const float* word, c
     if (n <= 0) return;
     check_ln_width(w);
     const long long rows = (long long)n * S;
-    bert_embed_ln_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, s>>>(ids, mask, word, pos, type0, gamma, beta, eps, n, S, w,
-                                                                   vocab, x, h, kv_len);
+    bert_embed_ln_kernel<false><<<(unsigned)((rows + 7) / 8), 256, 0, s>>>(ids, mask, word, pos, type0, gamma, beta, eps, n,
+                                                                          S, w, vocab, x, h, kv_len);
+    MB_CUDA(cudaGetLastError());
+}
+
+void mpnet_embed_ln(const int32_t* ids, const int32_t* mask, const float* word, const float* pos, const float* gamma,
+                    const float* beta, float eps, int n, int S, int w, int vocab, float* x, __nv_bfloat16* h,
+                    int32_t* kv_len, cudaStream_t s) {
+    if (n <= 0) return;
+    check_ln_width(w);
+    const long long rows = (long long)n * S;
+    bert_embed_ln_kernel<true><<<(unsigned)((rows + 7) / 8), 256, 0, s>>>(ids, mask, word, pos, nullptr, gamma, beta, eps, n,
+                                                                         S, w, vocab, x, h, kv_len);
     MB_CUDA(cudaGetLastError());
 }
 

@@ -30,6 +30,11 @@ void clip_text_embed(const int32_t* ids, const float* tok, const float* pos, int
 void bert_embed_ln(const int32_t* ids, const int32_t* mask, const float* word, const float* pos, const float* type0,
                    const float* gamma, const float* beta, float eps, int n, int S, int w, int vocab, float* x,
                    __nv_bfloat16* h, int32_t* kv_len, cudaStream_t s);
+// MPNet: x = LN(word[ids] + position[p]) with p = 2 + s for tokens (mask 1 or NULL) and p = 1 for pads; no token type.
+// kv_len as bert_embed_ln.  position: [>= S + 2, w].
+void mpnet_embed_ln(const int32_t* ids, const int32_t* mask, const float* word, const float* pos, const float* gamma,
+                    const float* beta, float eps, int n, int S, int w, int vocab, float* x, __nv_bfloat16* h,
+                    int32_t* kv_len, cudaStream_t s);
 
 // CLIP head: for image b take token row (b * S + row_in_seq[b]) (row_in_seq NULL -> 0), LayerNorm it, multiply by
 // proj [w, E] (fp32), optionally divide by the L2 norm (no epsilon: abstract_clip_model.py:83-85).

@@ -1,4 +1,4 @@
-// Encoder runtime: CLIP ViT image tower, CLIP text tower, BERT (e5) — SURVEY §8 a2-a5.
+// Encoder runtime: CLIP ViT image tower, CLIP text tower, BERT (e5), MPNet (all-mpnet-base-v2) — SURVEY §8 a2-a5.
 //
 // What the reference calls (third-party, restated in oracle/encoders.py):
 //   OPEN_CLIP.encode_image / encode_text   src/marqo/core/inference/embedding_models/open_clip_model.py:249-286
@@ -56,6 +56,8 @@ struct TowerW {
     // text / bert embeddings
     const float *tok = nullptr, *type0 = nullptr, *emb_ln_w = nullptr, *emb_ln_b = nullptr;
     int max_pos = 0;
+    // MPNet: relative-position bias folded to the attention kernels' table [heads, attention::REL_T] (log2 units)
+    const float* rel_bias = nullptr;
 };
 
 }  // namespace
@@ -198,7 +200,18 @@ void build_clip_layers(b200_model* m, TowerW& T, const std::string& prefix) {
     }
 }
 
-void build_bert_layers(b200_model* m, TowerW& T) {
+// HF parameter names of a post-LN layer below "encoder.layer.N.": BertLayer and MPNetLayer differ in the attention part
+struct PostLnNames {
+    const char* qkv[3];   // query / key / value Linear
+    const char* out;      // attention output Linear
+    const char* ln1;      // LayerNorm after attention
+};
+constexpr PostLnNames BERT_NAMES{{"attention.self.query", "attention.self.key", "attention.self.value"},
+                                 "attention.output.dense", "attention.output.LayerNorm"};
+constexpr PostLnNames MPNET_NAMES{{"attention.attn.q", "attention.attn.k", "attention.attn.v"}, "attention.attn.o",
+                                  "attention.LayerNorm"};
+
+void build_bert_layers(b200_model* m, TowerW& T, const PostLnNames& nm = BERT_NAMES) {
     const long long w = T.d.width, mlp = T.d.mlp;
     T.layers.resize(T.d.layers);
     for (int i = 0; i < T.d.layers; ++i) {
@@ -211,25 +224,24 @@ void build_bert_layers(b200_model* m, TowerW& T) {
         dev_alloc((void**)&bq, (size_t)3 * w * 4);
         m->owned.push_back(wq);
         m->owned.push_back(bq);
-        const char* names[3] = {"query", "key", "value"};
         for (int j = 0; j < 3; ++j) {
-            const std::string base = p + "attention.self." + names[j];
+            const std::string base = p + nm.qkv[j];
             kernels::f32_to_bf16(param(m, base + ".weight", w * w), wq + (size_t)j * w * w, w * w, m->stream);
             MB_CUDA(cudaMemcpyAsync(bq + (size_t)j * w, param(m, base + ".bias", w), (size_t)w * 4, cudaMemcpyDeviceToDevice,
                                     m->stream));
         }
         MB_CUDA(cudaStreamSynchronize(m->stream));
         for (int j = 0; j < 3; ++j) {
-            const std::string nm = p + "attention.self." + names[j] + ".weight";
-            cudaFree(m->raw[nm].p);
-            m->raw.erase(nm);
+            const std::string wn = p + nm.qkv[j] + ".weight";
+            cudaFree(m->raw[wn].p);
+            m->raw.erase(wn);
         }
         L.w_qkv = wq;
         L.b_qkv = bq;
-        L.w_o = to_bf16(m, p + "attention.output.dense.weight", w * w);
-        L.b_o = param(m, p + "attention.output.dense.bias", w);
-        L.ln1_w = param(m, p + "attention.output.LayerNorm.weight", w);  // post-LN after attention
-        L.ln1_b = param(m, p + "attention.output.LayerNorm.bias", w);
+        L.w_o = to_bf16(m, p + nm.out + ".weight", w * w);
+        L.b_o = param(m, p + nm.out + ".bias", w);
+        L.ln1_w = param(m, p + nm.ln1 + ".weight", w);  // post-LN after attention
+        L.ln1_b = param(m, p + nm.ln1 + ".bias", w);
         L.w_fc = to_bf16(m, p + "intermediate.dense.weight", mlp * w);
         L.b_fc = param(m, p + "intermediate.dense.bias", mlp);
         L.w_proj = to_bf16(m, p + "output.dense.weight", w * mlp);
@@ -273,9 +285,10 @@ void linear(b200_model* m, Counter& c, const __nv_bfloat16* A, int M, int K, con
     ++c.n;
 }
 
-void attend(b200_model* m, Counter& c, int B, int S, int w, int heads, int mask_mode, const int32_t* kv_len) {
+void attend(b200_model* m, Counter& c, int B, int S, int w, int heads, int mask_mode, const int32_t* kv_len,
+            const float* bias_log2 = nullptr) {
     ProfScope ps(m, 1);
-    c.n += attention::launch(m->qkv, m->o, B, S, w, heads, mask_mode, kv_len, m->stream);
+    c.n += attention::launch(m->qkv, m->o, B, S, w, heads, mask_mode, kv_len, bias_log2, m->stream);
 }
 
 // LayerNorm fused into the producing residual GEMM's epilogue (gemm.cuh: Epilogue::ln_*).  OFF by default: correct
@@ -371,11 +384,11 @@ void run_clip_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, i
     }
 }
 
-// Post-LN blocks (HF BertLayer); on entry x (fp32) and h (bf16) both hold the embedding LayerNorm output.  Both
-// LayerNorms of a layer run inside the epilogue of the GEMM before them and rewrite x in place.
-void run_bert_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S) {
+// Post-LN blocks (HF BertLayer / MPNetLayer); on entry x (fp32) and h (bf16) both hold the embedding LayerNorm output.
+// Both LayerNorms of a layer run inside the epilogue of the GEMM before them and rewrite x in place.  eps: 1e-12 for
+// BERT, 1e-5 for MPNet; T.rel_bias (MPNet) is added to every attention score.
+void run_bert_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, float eps) {
     const int M = B * S, w = T.d.width, mlp = T.d.mlp;
-    const float eps = 1e-12f;
     const int fmode = ln_fusion_mode();
     const bool fused = fmode != 0, fused_o = fmode == 1;
     for (const LayerW& L : T.layers) {
@@ -384,7 +397,7 @@ void run_bert_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S) {
         e1.out = m->qkv;
         e1.ldo = 3 * w;
         linear(m, c, m->h, M, w, L.w_qkv, 3 * w, e1);
-        attend(m, c, B, S, w, T.d.heads, attention::MASK_KEYLEN, m->aux);
+        attend(m, c, B, S, w, T.d.heads, attention::MASK_KEYLEN, m->aux, T.rel_bias);
         gemm::Epilogue e2;
         e2.bias = L.b_o;
         e2.residual = m->x;
@@ -423,6 +436,10 @@ void run_bert_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S) {
 }
 
 // images already as device uint8 [n, S, S, 3] (u8 != nullptr) or device fp32 CHW (f32 != nullptr)
+// MPNet's LayerNorm eps (layer_norm_eps of the all-mpnet-base-v2 family's config.json; transformers' MPNetConfig
+// default is 1e-12)
+constexpr float MPNET_LN_EPS = 1e-5f;
+
 void forward_images_eager(b200_model* m, Counter& c, const uint8_t* u8, const float* f32, int n, int normalize,
                           float* d_out) {
     const TowerW& T = m->vision;
@@ -478,11 +495,18 @@ void forward_tokens_eager(b200_model* m, Counter& c, const int32_t* d_ids, const
         kernels::clip_head(m->x, S, m->aux, T.ln_out_w, T.ln_out_b, 1e-5f, T.proj, n, w, m->desc.embed_dim, normalize,
                            d_out, m->pooled, m->stream);
         c.n += 3;
+    } else if (m->desc.arch == B200_ARCH_MPNET) {
+        kernels::mpnet_embed_ln(d_ids, d_mask, T.tok, T.pos, T.emb_ln_w, T.emb_ln_b, MPNET_LN_EPS, n, S, w, T.d.vocab,
+                                m->x, m->h, m->aux, m->stream);
+        c.n += 1;
+        run_bert_blocks(m, c, T, n, S, MPNET_LN_EPS);
+        kernels::bert_head(m->x, m->aux, n, S, w, m->desc.pool, normalize, d_out, m->stream);
+        c.n += 1;
     } else {
         kernels::bert_embed_ln(d_ids, d_mask, T.tok, T.pos, T.type0, T.emb_ln_w, T.emb_ln_b, 1e-12f, n, S, w, T.d.vocab,
                                m->x, m->h, m->aux, m->stream);
         c.n += 1;
-        run_bert_blocks(m, c, T, n, S);
+        run_bert_blocks(m, c, T, n, S, 1e-12f);
         kernels::bert_head(m->x, m->aux, n, S, w, m->desc.pool, normalize, d_out, m->stream);
         c.n += 1;
     }
@@ -624,7 +648,8 @@ int b200_model_create(int device, const b200_model_desc* desc, b200_model** out)
         int major = 0;
         MB_CUDA(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, device));
         if (major != 10) fail(B200_ERR_NO_DEVICE, "device %d has compute capability %d.x; sm_100 required", device, major);
-        MB_CHECK_ARG(desc->arch == B200_ARCH_CLIP || desc->arch == B200_ARCH_BERT, "unknown arch %d", desc->arch);
+        MB_CHECK_ARG(desc->arch == B200_ARCH_CLIP || desc->arch == B200_ARCH_BERT || desc->arch == B200_ARCH_MPNET,
+                     "unknown arch %d", desc->arch);
         MB_CHECK_ARG(desc->max_batch > 0, "max_batch must be positive");
         MB_CHECK_ARG(desc->embed_dim > 0 && desc->embed_dim <= 4096, "embed_dim out of range");
         const bool has_vision = desc->arch == B200_ARCH_CLIP && desc->vision.layers > 0;
@@ -641,6 +666,10 @@ int b200_model_create(int device, const b200_model_desc* desc, b200_model** out)
             MB_CHECK_ARG(desc->text.ctx > 0 && desc->text.vocab > 0, "text.ctx and text.vocab must be positive");
             if (desc->arch == B200_ARCH_BERT)
                 MB_CHECK_ARG(desc->embed_dim == desc->text.width, "BERT embed_dim must equal width");
+            if (desc->arch == B200_ARCH_MPNET) {
+                MB_CHECK_ARG(desc->embed_dim == desc->text.width, "MPNet embed_dim must equal width");
+                MB_CHECK_ARG(desc->text.ctx > 2, "MPNet text.ctx (max_position_embeddings) must exceed 2");
+            }
         }
         DeviceGuard g(device);
         b200_model* m = new b200_model();
@@ -750,6 +779,24 @@ int b200_model_finalize(b200_model* m) {
                 T.ln_out_w = param(m, "ln_final.weight", w);
                 T.ln_out_b = param(m, "ln_final.bias", w);
                 T.proj = param(m, "text_projection", w * E);
+            } else if (m->desc.arch == B200_ARCH_MPNET) {
+                T.max_pos = T.d.ctx - 2;   // position ids 2 .. S + 1
+                T.tok = param(m, "embeddings.word_embeddings.weight", (long long)T.d.vocab * w);
+                T.pos = param(m, "embeddings.position_embeddings.weight", (long long)T.d.ctx * w);
+                T.emb_ln_w = param(m, "embeddings.LayerNorm.weight", w);
+                T.emb_ln_b = param(m, "embeddings.LayerNorm.bias", w);
+                build_bert_layers(m, T, MPNET_NAMES);
+                // [32 buckets, heads] -> the attention kernels' per-head rows over d = key - query (host fold)
+                const int H = T.d.heads;
+                const float* rb = param(m, "encoder.relative_attention_bias.weight", (long long)attention::REL_BUCKETS * H);
+                std::vector<float> rel((size_t)attention::REL_BUCKETS * H), folded((size_t)H * attention::REL_T);
+                MB_CUDA(cudaMemcpy(rel.data(), rb, rel.size() * 4, cudaMemcpyDeviceToHost));
+                attention::fold_relative_bias(rel.data(), H, T.max_pos - 1, folded.data());
+                float* tbl = nullptr;
+                dev_alloc((void**)&tbl, folded.size() * 4);
+                m->owned.push_back(tbl);
+                MB_CUDA(cudaMemcpy(tbl, folded.data(), folded.size() * 4, cudaMemcpyHostToDevice));
+                T.rel_bias = tbl;
             } else {
                 T.tok = param(m, "embeddings.word_embeddings.weight", (long long)T.d.vocab * w);
                 T.pos = param(m, "embeddings.position_embeddings.weight", (long long)T.d.ctx * w);
@@ -841,7 +888,7 @@ int b200_model_encode_tokens(b200_model* m, const int32_t* ids, const int32_t* a
         require_ready(m);
         MB_CHECK_ARG(ids && out, "NULL buffer");
         check_tokens_args(m, n, seq);
-        if (attn_mask && m->desc.arch == B200_ARCH_BERT) {
+        if (attn_mask && (m->desc.arch == B200_ARCH_BERT || m->desc.arch == B200_ARCH_MPNET)) {
             // the kernels implement prefix (right-padded) masks, which is what the tokenizer call at
             // hugging_face_model.py:179-185 produces
             for (int b = 0; b < n; ++b) {

@@ -289,12 +289,14 @@ def _to_numpy_f32(t) -> np.ndarray:
 
 
 class Encoder:
-    """A CLIP (vision + text towers) or BERT encoder resident on one GPU.
+    """A CLIP (vision + text towers), BERT or MPNet encoder resident on one GPU.
 
     `config` keys — CLIP: embed_dim, act ("gelu"|"quickgelu"), mean, std, vision{width,layers,heads,mlp,patch,
     image_size}, text{width,layers,heads,mlp,ctx,vocab};  BERT: width, layers, heads, mlp, vocab, max_pos, type_vocab,
-    pool ("mean"|"cls").  `weights` maps checkpoint parameter names (open_clip state_dict names / HF BertModel names) to
-    fp32 arrays or torch tensors.
+    pool ("mean"|"cls");  MPNet: as BERT without type_vocab, max_pos = max_position_embeddings (514: sequences of up to
+    512 tokens), optional buckets (32) and ln_eps (1e-5), the only values the library implements.  `weights` maps
+    checkpoint parameter names (open_clip state_dict names / HF BertModel / MPNetModel names) to fp32 arrays or torch
+    tensors.
     """
 
     def __init__(self, arch: str, config: dict, weights: dict, device: int = 0, max_batch: int = 256):
@@ -326,6 +328,15 @@ class Encoder:
             d.type_vocab = int(config.get("type_vocab", 2))
             d.text = N.TowerDesc(config["width"], config["layers"], config["heads"], config["mlp"],
                                  config.get("max_pos", 512), config["vocab"], 0, 0)
+            self.image_size = 0
+        elif arch == "mpnet":
+            if int(config.get("buckets", 32)) != 32 or float(config.get("ln_eps", 1e-5)) != 1e-5:
+                raise ValueError("MPNet: only 32 relative-position buckets and LayerNorm eps 1e-5 are implemented")
+            d.arch = N.ARCH_MPNET
+            d.embed_dim = int(config["width"])
+            d.pool = N.POOL_CLS if config.get("pool", "mean") == "cls" else N.POOL_MEAN
+            d.text = N.TowerDesc(config["width"], config["layers"], config["heads"], config["mlp"],
+                                 config.get("max_pos", 514), config["vocab"], 0, 0)
             self.image_size = 0
         else:
             raise ValueError(f"unknown arch {arch!r}")
@@ -529,6 +540,26 @@ def debug_attention(qkv, B: int, S: int, W: int, H: int, mask: int = 0, kv_len=N
     kl = None if kv_len is None else _as(kv_len, np.int32)
     out = np.empty((B * S, W), np.float32)
     N.check(N.load().b200_debug_attention(device, _ptr(q), B, S, W, H, mask, _ptr(kl), _ptr(out)))
+    return out
+
+
+def debug_attention_relbias(qkv, B: int, S: int, W: int, H: int, rel_bias, mask: int = 0, kv_len=None,
+                            device: int = 0) -> np.ndarray:
+    """debug_attention with MPNet's relative-position bias rel_bias [32, H] (checkpoint layout) added to the scores."""
+    q = _as(qkv, np.float32)
+    rb = _as(rel_bias, np.float32)
+    if rb.shape != (32, H):
+        raise ValueError(f"expected rel_bias [32, {H}], got {rb.shape}")
+    kl = None if kv_len is None else _as(kv_len, np.int32)
+    out = np.empty((B * S, W), np.float32)
+    N.check(N.load().b200_debug_attention_relbias(device, _ptr(q), B, S, W, H, mask, _ptr(kl), _ptr(rb), _ptr(out)))
+    return out
+
+
+def relative_position_buckets(max_distance: int) -> np.ndarray:
+    """The library's relative-position bucket of every d = key - query in [-max_distance, max_distance] (host only)."""
+    out = np.empty(2 * max_distance + 1, np.int32)
+    N.check(N.load().b200_debug_relative_position_buckets(int(max_distance), _ptr(out)))
     return out
 
 

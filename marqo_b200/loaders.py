@@ -32,7 +32,9 @@ def _resolve_weights(props: dict, arch: dict, kind: str) -> Dict[str, np.ndarray
     w = props.get("weights")
     if w is None and props.get("random_init") is not None:
         seed = int(props["random_init"])
-        return weights_mod.random_clip_weights(arch, seed) if kind == "clip" else weights_mod.random_bert_weights(arch, seed)
+        random = {"clip": weights_mod.random_clip_weights, "bert": weights_mod.random_bert_weights,
+                  "mpnet": weights_mod.random_mpnet_weights}[kind]
+        return random(arch, seed)
     if w is None:
         raise ModelLoadError("model_properties needs `weights` (state dict or checkpoint path) or `random_init`; "
                              "checkpoint download is Marqo's job (open_clip_model.py:107-131) and out of scope here")
@@ -40,6 +42,8 @@ def _resolve_weights(props: dict, arch: dict, kind: str) -> Dict[str, np.ndarray
         w = weights_mod.load_state_dict(w)
     if kind == "bert":
         w = weights_mod.strip_hf_prefix(w)
+    elif kind == "mpnet":
+        w = weights_mod.strip_hf_prefix(w, "mpnet.")
     return w
 
 
@@ -284,15 +288,19 @@ class B200HuggingFace:
         if props.get("poolingMethod") or props.get("pooling_method"):  # hugging_face_model_properties.py
             arch = dict(arch, pool=(props.get("poolingMethod") or props.get("pooling_method")))
         self.arch = arch
-        self._model = Encoder("bert", arch, _resolve_weights(props, arch, "bert"), device=_validate_device(self.device),
+        kind = arch.get("family", "bert")   # "bert" (e5 & co.) or "mpnet" (all-mpnet-base & co.)
+        self._model = Encoder(kind, arch, _resolve_weights(props, arch, kind), device=_validate_device(self.device),
                               max_batch=int(props.get("max_batch", 256)))
         self._tokenizer = props.get("tokenizer") or self._default_tokenizer()
 
     def _default_tokenizer(self):
         if self.model_properties.get("vocab_file"):
             from .tokenizers import WordPieceTokenizer
+            specials = {}
+            if self.arch.get("family") == "mpnet":   # MPNetTokenizer: WordPiece framed by <s> ... </s>, <pad> id 1
+                specials = dict(cls_token="<s>", sep_token="</s>", pad_token="<pad>", unk_token="[UNK]")
             return WordPieceTokenizer(self.model_properties["vocab_file"],
-                                      do_lower_case=bool(self.model_properties.get("do_lower_case", True)))
+                                      do_lower_case=bool(self.model_properties.get("do_lower_case", True)), **specials)
         try:
             from transformers import AutoTokenizer
             return AutoTokenizer.from_pretrained(self.model_properties["name"])

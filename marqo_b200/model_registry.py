@@ -1,7 +1,8 @@
 """Model name -> properties + architecture for the models the engine serves.
 
 Property dicts (`name`, `dimensions`, `type`, `tokens`, prefixes) are the reference's registry entries
-(src/marqo/s2_inference/model_registry.py:142-231 for open_clip/*, :771-788 for hf/e5-*); `type` is rewritten to the
+(src/marqo/s2_inference/model_registry.py:142-231 for open_clip/*, :771-788 for hf/e5-*, :630-641 and :668-679 for the
+MPNet sentence encoders); `type` is rewritten to the
 engine's loader types ("b200_open_clip" / "b200_hf") so that both engines can be registered side by side in
 MODEL_PROPERTIES['loaders'] (model_registry.py:2133-2145).  The `arch` blocks are the shapes that live in
 open_clip 2.24.0 `model_configs/*.json` and the HF `config.json` files (SURVEY.md §8)."""
@@ -28,6 +29,12 @@ def _clip_arch(embed, vw, vl, vh, patch, tw, tl, th, act="gelu"):
 def _bert_arch(w, layers, heads, pool="mean"):
     return {"width": w, "layers": layers, "heads": heads, "mlp": 4 * w, "vocab": 30522, "max_pos": 512,
             "type_vocab": 2, "pool": pool}
+
+
+def _mpnet_arch(pool="mean"):
+    # HF MPNetModel config.json of the all-mpnet-base / all_datasets_*_mpnet-base checkpoints
+    return {"family": "mpnet", "width": 768, "layers": 12, "heads": 12, "mlp": 3072, "vocab": 30527, "max_pos": 514,
+            "buckets": 32, "ln_eps": 1e-5, "pool": pool}
 
 
 _VIT_B_32 = dict(embed=512, vw=768, vl=12, vh=12, patch=32, tw=512, tl=12, th=8)
@@ -64,6 +71,12 @@ def _models() -> Dict[str, dict]:
         m[f"hf/{short}"] = {"name": repo, "dimensions": w, "tokens": 512, "type": TYPE_HF, "model_size": size,
                             "text_query_prefix": "query: ", "text_chunk_prefix": "passage: ", "notes": "",
                             "arch": _bert_arch(w, layers, heads)}
+    for short, repo in (("all-mpnet-base-v1", "sentence-transformers/all-mpnet-base-v1"),
+                        ("all-mpnet-base-v2", "sentence-transformers/all-mpnet-base-v2"),
+                        ("all_datasets_v3_mpnet-base", "flax-sentence-embeddings/all_datasets_v3_mpnet-base"),
+                        ("all_datasets_v4_mpnet-base", "flax-sentence-embeddings/all_datasets_v4_mpnet-base")):
+        m[f"hf/{short}"] = {"name": repo, "dimensions": 768, "tokens": 128, "type": TYPE_HF, "notes": "",
+                            "arch": _mpnet_arch()}
     return m
 
 

@@ -64,10 +64,16 @@ def _read(path_or_bytes: Union[str, Path, bytes]) -> bytes:
 
 
 class WordPieceTokenizer(_Tokenizer):
-    def __init__(self, vocab: Union[str, Path, bytes], do_lower_case: bool = True, model_max_length: int = 512):
+    """BERT's special tokens by default; MPNet's tokenizer is cls_token="<s>", sep_token="</s>", pad_token="<pad>",
+    unk_token="[UNK]"."""
+
+    def __init__(self, vocab: Union[str, Path, bytes], do_lower_case: bool = True, model_max_length: int = 512,
+                 cls_token: str = "[CLS]", sep_token: str = "[SEP]", pad_token: str = "[PAD]", unk_token: str = "[UNK]"):
         data = _read(vocab)
         h = C.c_void_p()
-        N.check(N.load().b200_tokenizer_create_wordpiece(data, len(data), 1 if do_lower_case else 0, C.byref(h)))
+        N.check(N.load().b200_tokenizer_create_wordpiece_special(
+            data, len(data), 1 if do_lower_case else 0, cls_token.encode(), sep_token.encode(), pad_token.encode(),
+            unk_token.encode(), C.byref(h)))
         super().__init__(h)
         self.model_max_length = model_max_length
 

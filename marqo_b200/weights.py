@@ -1,7 +1,7 @@
 """Checkpoint plumbing for the encoders: state-dict loading and random initialisation.
 
 The engine consumes parameters under their checkpoint names (open_clip state_dict names for CLIP, HF BertModel names
-for BERT), so a real checkpoint loads unchanged: open_clip `*.pt/*.bin` state dicts, HF `pytorch_model.bin`, or an
+for BERT, HF MPNetModel names for MPNet), so a real checkpoint loads unchanged: open_clip `*.pt/*.bin` state dicts, HF `pytorch_model.bin`, or an
 `.npz` with the same keys.  `random_*` build seeded random-init weights of a given architecture (bench.py and the
 service's self-test use them — there is no network for real checkpoints in the build environment)."""
 from __future__ import annotations
@@ -32,10 +32,11 @@ def load_state_dict(path: str) -> Dict[str, np.ndarray]:
     return out
 
 
-def strip_hf_prefix(sd: Dict[str, np.ndarray]) -> Dict[str, np.ndarray]:
-    """HF checkpoints saved from BertForXxx carry a 'bert.' prefix; BertModel checkpoints do not."""
-    if any(k.startswith("bert.") for k in sd):
-        return {k[len("bert."):]: v for k, v in sd.items() if k.startswith("bert.")}
+def strip_hf_prefix(sd: Dict[str, np.ndarray], prefix: str = "bert.") -> Dict[str, np.ndarray]:
+    """HF checkpoints saved from BertForXxx / MPNetForXxx carry a 'bert.' / 'mpnet.' prefix; BertModel and MPNetModel
+    checkpoints do not."""
+    if any(k.startswith(prefix) for k in sd):
+        return {k[len(prefix):]: v for k, v in sd.items() if k.startswith(prefix)}
     return sd
 
 
@@ -121,4 +122,32 @@ def random_bert_weights(arch: dict, seed: int = 1234) -> Dict[str, np.ndarray]:
         sd[p + "output.dense.bias"] = _vec(g, w)
         sd[p + "output.LayerNorm.weight"] = _vec(g, w, 0.1, 1.0)
         sd[p + "output.LayerNorm.bias"] = _vec(g, w)
+    return sd
+
+
+def random_mpnet_weights(arch: dict, seed: int = 1234) -> Dict[str, np.ndarray]:
+    """Seeded random weights under HF MPNetModel parameter names (relative-attention bias [32, heads] included)."""
+    g = _rng(seed)
+    w, mlp = arch["width"], arch["mlp"]
+    sd: Dict[str, np.ndarray] = {}
+    sd["embeddings.word_embeddings.weight"] = g.standard_normal((arch["vocab"], w), dtype=np.float32)
+    sd["embeddings.position_embeddings.weight"] = 0.5 * g.standard_normal((arch.get("max_pos", 514), w), dtype=np.float32)
+    sd["embeddings.LayerNorm.weight"] = _vec(g, w, 0.1, 1.0)
+    sd["embeddings.LayerNorm.bias"] = _vec(g, w)
+    for i in range(arch["layers"]):
+        p = f"encoder.layer.{i}."
+        for nm in ("q", "k", "v"):
+            sd[p + f"attention.attn.{nm}.weight"] = _lin(g, w, w, 1.5)
+            sd[p + f"attention.attn.{nm}.bias"] = _vec(g, w)
+        sd[p + "attention.attn.o.weight"] = _lin(g, w, w)
+        sd[p + "attention.attn.o.bias"] = _vec(g, w)
+        sd[p + "attention.LayerNorm.weight"] = _vec(g, w, 0.1, 1.0)
+        sd[p + "attention.LayerNorm.bias"] = _vec(g, w)
+        sd[p + "intermediate.dense.weight"] = _lin(g, mlp, w)
+        sd[p + "intermediate.dense.bias"] = _vec(g, mlp)
+        sd[p + "output.dense.weight"] = _lin(g, w, mlp)
+        sd[p + "output.dense.bias"] = _vec(g, w)
+        sd[p + "output.LayerNorm.weight"] = _vec(g, w, 0.1, 1.0)
+        sd[p + "output.LayerNorm.bias"] = _vec(g, w)
+    sd["encoder.relative_attention_bias.weight"] = _vec(g, 32 * arch["heads"], 1.0).reshape(32, arch["heads"])
     return sd
