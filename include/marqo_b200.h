@@ -397,13 +397,6 @@ int b200_jpeg_decode_batch(int device, const uint8_t* const* files, const size_t
  * the residual buffer, as in the model's out_proj / fc2, which add onto the residual stream they overwrite. */
 int b200_debug_gemm(int device, const float* A, const float* W, const float* bias, const float* residual, int M, int N,
                     int K, int act, int out_bf16, int in_place, float* out);
-/* Residual GEMM with the LayerNorm fused into its epilogue (gemm.cuh Epilogue::ln_*): out_x fp32 [M,N] = A W^T + bias
- * (+ residual); out_ln = LayerNorm(out_x) * gamma + beta rounded to bf16 (returned as fp32).  in_place != 0: the fp32
- * normalised rows also replace out_x (BERT post-LN).  The launch is repeated `repeats` times, alternating between two strip
- * counter arrays as the model's out_proj / fc2 do; with in_place == 0 every repeat computes the same thing. */
-int b200_debug_gemm_ln(int device, const float* A, const float* W, const float* bias, const float* residual, int M, int N,
-                       int K, const float* gamma, const float* beta, float eps, int in_place, int repeats, float* out_x,
-                       float* out_ln);
 /* ViT patch embedding of uint8 HWC images [n,S,S,3]: ToTensor + Normalize (mean3/std3) -> conv1 (conv_w fp32
  * [N, 3*patch*patch], no bias) -> token rows: out fp32 [n*(G+1), N], row b*(G+1)+1+i = patch i of image b (+ pos[1+i]
  * when pos != NULL), class-token rows left zero.  use_gather != 0: the fused gather GEMM (no patch matrix in HBM,

@@ -108,7 +108,6 @@ _SIGNATURES = {
     "b200_model_profile": (C.c_int, [_P, C.POINTER(C.c_float), C.POINTER(C.c_int), C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "b200_model_last_timing": (C.c_int, [_P, C.POINTER(C.c_float), C.POINTER(C.c_int)]),
     "b200_debug_gemm": (C.c_int, [C.c_int, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
-    "b200_debug_gemm_ln": (C.c_int, [C.c_int, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, _P, _P, C.c_float, C.c_int, C.c_int, _P, _P]),
     "b200_debug_patch_embed": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int, _P, _P, _P, C.c_int, _P]),
     "b200_debug_attention": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
     "b200_debug_attention_relbias": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),

@@ -1,7 +1,7 @@
 // Multi-head attention over packed QKV (head_dim 64), flash-style online softmax in fp32.
-//   S >= 128: tcgen05 / TMEM kernel (attention_tc.cu) — 128 x 128 tiles, TMA-fed, thread-per-row softmax.
-//   S <  128: 64-row warp-level kernel (attention.cu, mma.sync m16n8k16) — short sequences would leave most of a
-//             128-wide tcgen05 tile masked.
+//   129 <= S <= 257 without a bias: one-shot tcgen05 kernel (attention_os.cu) — all keys in one MMA.
+//   every other input: tcgen05 / TMEM block kernel (attention_tc.cu) — 128 x 128 tiles, TMA-fed, thread-per-row
+//             softmax; S < 128 packs several sequences into one tile under a block-diagonal mask.
 #pragma once
 #include "common.cuh"
 

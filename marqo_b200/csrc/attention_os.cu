@@ -22,7 +22,6 @@
 //   warp 6  the remainder QUERY row (mma.sync against the K / V tiles while they sit in shared memory), once per
 //           (batch, head), as soon as the tiles have landed
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #include "attention.cuh"
@@ -145,7 +144,7 @@ __global__ void __launch_bounds__(THREADS, 2)
 attention_os_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_tail,
                     const __nv_bfloat16* __restrict__ qkv,
                     __nv_bfloat16* __restrict__ out, int S, int W, int H, const int32_t* __restrict__ kv_len,
-                    float scale_log2e, int s_main, int has_tail, int total_units, int reverse) {
+                    float scale_log2e, int s_main, int has_tail, int total_units) {
     extern __shared__ __align__(1024) uint8_t smem[];
     uint8_t* sQ = smem;                         // two 16 KB tiles
     uint8_t* sK = sQ + 2 * Q_BYTES;             // 256 keys x 64 dims, K-major 128B-swizzled (two TMA boxes)
@@ -244,13 +243,14 @@ attention_os_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_const
     };
 
     // every role walks units u = blockIdx.x, + gridDim.x, ... (unit = (batch, head)) and the unit's two query blocks;
-    // n = items (query blocks) done so far, uc = units done so far
+    // n = items (query blocks) done so far, uc = units done so far.  Unit u is (batch, head) ur = total_units - 1 - u:
+    // the QKV GEMM wrote the packed qkv matrix in ascending row order, so its last rows are the ones still in L2.
     if (warp == 0) {
         // ================================================================== TMA producer
         if (lane == 0) {
             uint32_t n = 0, uc = 0;
             for (int u = blockIdx.x; u < total_units; u += gridDim.x, ++uc) {
-                const int ur = reverse ? total_units - 1 - u : u;
+                const int ur = total_units - 1 - u;
                 const int b = ur / H, h = ur - b * H;
                 const int row_base = b * S;
                 for (int qb = 0; qb < q_blocks; ++qb, ++n) {
@@ -296,7 +296,7 @@ attention_os_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_const
         const size_t ld = (size_t)3 * W;
         const int gq = lane >> 2, tq = lane & 3;
         for (int u = blockIdx.x; u < total_units; u += gridDim.x, ++uc) {
-            const int ur = reverse ? total_units - 1 - u : u;
+            const int ur = total_units - 1 - u;
             const int b = ur / H, h = ur - b * H;
             const int row_base = b * S;
             int len = S;
@@ -305,7 +305,7 @@ attention_os_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_const
                 // (the remainder KEY is the tensor core's job: a 16-row K tile + a 16-column MMA per item, see the MMA warp)
                 const int nu = u + gridDim.x;
                 if (has_tail && lane == 0 && nu < total_units) {   // the next unit's remainder row: into L2 ahead of time
-                    const int nur = reverse ? total_units - 1 - nu : nu;
+                    const int nur = total_units - 1 - nu;
                     const int nb = nur / H, nh = nur - nb * H;
                     const __nv_bfloat16* nrow = qkv + ((size_t)nb * S + s_main) * ld + nh * HD;
                     asm volatile("prefetch.global.L2 [%0];" ::"l"(nrow));
@@ -461,7 +461,7 @@ attention_os_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_const
         const uint32_t lane_addr = tmem_base + (uint32_t(sp * 32) << 16);
         uint32_t n = 0;
         for (int u = blockIdx.x; u < total_units; u += gridDim.x) {
-            const int ur = reverse ? total_units - 1 - u : u;
+            const int ur = total_units - 1 - u;
             const int b = ur / H, h = ur - b * H;
             const int row_base = b * S;
             int len = S;
@@ -585,8 +585,7 @@ attention_os_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_const
 }  // namespace os
 
 bool os_supported(int S, int mask) {
-    static const bool disabled = getenv("MARQO_B200_ATTN_NO_ONESHOT") != nullptr;   // A/B timing switch
-    return !disabled && S > os::BQ && S <= os::NK + 1 && (mask == MASK_NONE || mask == MASK_KEYLEN);
+    return S > os::BQ && S <= os::NK + 1 && (mask == MASK_NONE || mask == MASK_KEYLEN);
 }
 
 int launch_os(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W, int H, int mask, const int32_t* kv_len,
@@ -613,15 +612,12 @@ int launch_os(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W,
     const int s_main = tail ? os::NK : S;
     const int total_units = B * H;
     const int grid = std::min(2 * sm_count(device), total_units);
-    // (batch, head) units are walked from the LAST sequence to the first: the QKV GEMM wrote the packed qkv matrix in
-    // ascending row order, so its last rows are the ones still in L2; MARQO_B200_ATTN_FORWARD=1 restores the forward order
-    static const int reverse = getenv("MARQO_B200_ATTN_FORWARD") == nullptr ? 1 : 0;
     if (mask == MASK_NONE)
         os::attention_os_kernel<MASK_NONE><<<grid, os::THREADS, os::SMEM_BYTES, stream>>>(
-            tmap, tmap_tail, qkv, out, S, W, H, kv_len, scale_log2e, s_main, tail ? 1 : 0, total_units, reverse);
+            tmap, tmap_tail, qkv, out, S, W, H, kv_len, scale_log2e, s_main, tail ? 1 : 0, total_units);
     else
         os::attention_os_kernel<MASK_KEYLEN><<<grid, os::THREADS, os::SMEM_BYTES, stream>>>(
-            tmap, tmap_tail, qkv, out, S, W, H, kv_len, scale_log2e, s_main, tail ? 1 : 0, total_units, reverse);
+            tmap, tmap_tail, qkv, out, S, W, H, kv_len, scale_log2e, s_main, tail ? 1 : 0, total_units);
     MB_CUDA(cudaGetLastError());
     return 1;
 }

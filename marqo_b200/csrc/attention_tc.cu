@@ -8,9 +8,10 @@
 // packed qkv matrix).  Warp 1: single-thread tcgen05.mma issuer:
 //   S = Q K_j^T   (M=128, N=128, K=64;  A, B K-major)          -> TMEM columns [0,128)
 //   O += P_j V_j  (M=128, N=64,  K=128; A = P K-major from smem, B = V MN-major as loaded)  -> TMEM columns [128,192)
-// Warps 2-5: softmax, ONE THREAD PER QUERY ROW (TMEM lane == row): two passes over the row's 128 scores in TMEM
-// (max, then exp2 / sum / bf16 P written to smem in the UMMA K-major swizzled layout), running-max rescale of the O
-// accumulator through tcgen05.ld/st, final 1/l scaling and the bf16 store.  S of block g + 1 is issued before P.V of
+// Warps 2-5: softmax, ONE THREAD PER QUERY ROW (TMEM lane == row): one pass over the row's 128 scores in TMEM against a
+// lazy exponent reference (exp2 / sum / bf16 P written to smem in the UMMA K-major swizzled layout, the exact maximum
+// tracked on the side; a warp whose reference falls too far behind redoes the block exactly), rescale of the O
+// accumulator through tcgen05.ld/st when the reference moves, final 1/l scaling and the bf16 store.  S of block g + 1 is issued before P.V of
 // block g (also across items), so the next scores are ready when the softmax warps come back.
 // Warp 6: the remainder key and query row of a sequence such as 257 = 2 * 128 + 1 (ViT class token): the key's scores
 // against the 128 rows of the item and its V row are staged in smem for the epilogue; the row runs on mma.sync
@@ -19,7 +20,6 @@
 // BIAS (MPNet): a learned relative-position bias per (head, key - query) enters every score before the softmax; warp 6
 // stages the item's head row of the bias in shared memory instead of handling a remainder key / row.
 #include <algorithm>
-#include <cstdlib>
 #include <mutex>
 
 #include "attention.cuh"
@@ -51,7 +51,6 @@ constexpr uint32_t SMEM_BYTES_BIAS = Q_BYTES + KV_STAGES * 2 * KV_TILE_BYTES + P
 static_assert(SMEM_BYTES_BIAS <= 115712, "two CTAs per SM");
 constexpr uint32_t TMEM_COLS = 256;
 constexpr uint32_t S_COL = 0, O_COL = 128;
-constexpr int DEFAULT_SOFTMAX_MODE = 1;
 
 __device__ __forceinline__ float ex2(float x) {
     float y;
@@ -90,65 +89,12 @@ __device__ __forceinline__ void tmem_ld_wait_regs(uint32_t (&v)[32]) {
                  : "memory");
 }
 
-__device__ __forceinline__ void tmem_ld_wait_regs16(uint32_t (&v)[16]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]),
-                   "+r"(v[8]), "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15])
-                 :
-                 : "memory");
-}
-
 // Relative-position bias of key - query = d (log2 units): sB points at the staged head row's d = 0 entry.
 __device__ __forceinline__ float rel_bias(const float* sB, int d) { return sB[min(max(d, -REL_D), REL_D)]; }
 
-// 16 keys (block-local columns k0 .. k0 + 15) of a score row with FOUR independent sum / max chains: the softmax warps
-// are latency-bound (two of them per scheduler), so the serial `lsum += p` chain of the 32-key version below costs
-// more than its instructions.
-// BIAS: the scores are x = s * scale_log2e + bias (dk = block key 0 - query) and mx tracks x, not the raw s.
-template <bool FULL, bool BIAS = false>
-__device__ __forceinline__ void softmax_half_chunk(const uint32_t (&v)[16], int k0, int klo, int khi, float scale_log2e,
-                                                   float m_safe, float (&ls)[4], float (&mx)[4], uint8_t* sP, int r,
-                                                   const float* sB = nullptr, int dk = 0) {
-    uint32_t pk[8];
-#pragma unroll
-    for (int i = 0; i < 16; i += 2) {
-        const float s0 = __uint_as_float(v[i]), s1 = __uint_as_float(v[i + 1]);
-        float p0, p1;
-        const int a = (i >> 1) & 3;
-        if constexpr (BIAS) {
-            const int kk = k0 + i;
-            const float x0 = fmaf(s0, scale_log2e, rel_bias(sB, dk + kk));
-            const float x1 = fmaf(s1, scale_log2e, rel_bias(sB, dk + kk + 1));
-            const bool ok0 = FULL || (kk >= klo && kk < khi), ok1 = FULL || (kk + 1 >= klo && kk + 1 < khi);
-            mx[a] = ok0 ? fmaxf(mx[a], x0) : mx[a];
-            mx[a] = ok1 ? fmaxf(mx[a], x1) : mx[a];
-            p0 = ok0 ? ex2(x0 - m_safe) : 0.f;
-            p1 = ok1 ? ex2(x1 - m_safe) : 0.f;
-        } else if (FULL) {
-            mx[a] = fmaxf(mx[a], fmaxf(s0, s1));
-            p0 = ex2(fmaf(s0, scale_log2e, -m_safe));
-            p1 = ex2(fmaf(s1, scale_log2e, -m_safe));
-        } else {
-            const int kk = k0 + i;
-            const bool ok0 = kk >= klo && kk < khi, ok1 = kk + 1 >= klo && kk + 1 < khi;
-            mx[a] = ok0 ? fmaxf(mx[a], s0) : mx[a];
-            mx[a] = ok1 ? fmaxf(mx[a], s1) : mx[a];
-            p0 = ok0 ? ex2(fmaf(s0, scale_log2e, -m_safe)) : 0.f;
-            p1 = ok1 ? ex2(fmaf(s1, scale_log2e, -m_safe)) : 0.f;
-        }
-        ls[a] += p0 + p1;
-        pk[i >> 1] = pack2(p0, p1);
-    }
-    // keys k0 .. k0+15 -> 64-key chunk (k0 >> 6), 16-byte units ((k0 & 63) >> 3) and the next one, of row r
-    uint8_t* rowp = sP + (size_t)(k0 >> 6) * (BQ * 128) + (size_t)r * 128;
-    const int unit = (k0 & 63) >> 3;
-    *reinterpret_cast<uint4*>(rowp + ((unit ^ (r & 7)) << 4)) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-    *reinterpret_cast<uint4*>(rowp + (((unit + 1) ^ (r & 7)) << 4)) = make_uint4(pk[4], pk[5], pk[6], pk[7]);
-}
-
 // One 32-key chunk of a score row: p = exp2(s * scale - m_safe) for the keys in [klo, khi) (block-local indices), 0 for
 // the others; running raw maximum, row sum, bf16 P into the K-major 128B-swizzled A-operand layout.
-// BIAS: as softmax_half_chunk.
+// BIAS: the scores are x = s * scale_log2e + bias (dk = block key 0 - query) and mx tracks x, not the raw s.
 template <bool FULL, bool BIAS = false>
 __device__ __forceinline__ void softmax_chunk(const uint32_t (&v)[32], int c, int klo, int khi, float scale_log2e,
                                               float m_safe, float& lsum, float& mx, uint8_t* sP, int r,
@@ -229,12 +175,10 @@ __device__ __forceinline__ void item_extent(const Item& w, int S, int s_main, co
 // Two CTAs per SM: 14 warps over 4 schedulers put 4 warps on one of them, and a scheduler's register partition
 // (16384 registers) holds 4 warps only up to 128 registers each — a 144-register build (tried in round 2) silently
 // dropped to ONE CTA per SM and ran 1.85x slower.
-// SM: softmax schedule of the row threads — 0 two passes over S (exact block maximum), 1 one pass / one register buffer,
-// 2 one pass with the next chunk's tcgen05.ld in flight (two buffers).  All three use the lazy exponent reference.
 // BIAS: every score gets the relative-position bias of its head and of key - query (positions within the sequence, also
 // in packed tiles) before the softmax; warp 6 stages the item's head row of bias_log2 [H, REL_T] in shared memory
 // instead of handling a remainder key / row (the launcher never passes one).
-template <int MASK, bool PACKED, int SM, bool BIAS>
+template <int MASK, bool PACKED, bool BIAS>
 __global__ void __launch_bounds__(THREADS, 2)
 attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat16* __restrict__ qkv,
                     __nv_bfloat16* __restrict__ out, int S, int W, int H, const int32_t* __restrict__ kv_len,
@@ -683,122 +627,53 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
                 // warp-uniform (__any_sync): tcgen05.ld / st are warp-collective.
                 float lsum = 0.f, mx = -INFINITY, alpha = 1.f, m_new = m_run;
                 uint32_t va[32];
-                if (SM == 0) {
-                    // ---- two passes over S in TMEM: exact block maximum first, then exp / sum / P
+                // ---- one pass: reference = running reference (first block: max of the row's first 32 scores); the
+                //      exact maximum is tracked on the side and only checked afterwards
+                ptx::tmem_ld_32x32b_x32(lane_addr + S_COL, va);
+                tmem_ld_wait_regs(va);
+                float m_ref = m_run;
+                if (j == 0) {
+                    float c0 = -INFINITY;
+                    if constexpr (BIAS) {
+#pragma unroll
+                        for (int i = 0; i < 32; ++i)
+                            if (full || (i >= klo && i < khi))
+                                c0 = fmaxf(c0, fmaf(__uint_as_float(va[i]), scale_log2e, rel_bias(sB, dk + i)));
+                        m_ref = c0;
+                    } else {
+#pragma unroll
+                        for (int i = 0; i < 32; ++i)
+                            if (full || (i >= klo && i < khi)) c0 = fmaxf(c0, __uint_as_float(va[i]));
+                        m_ref = c0 * scale_log2e;
+                    }
+                }
+                const float m_safe = m_ref == -INFINITY ? 0.f : m_ref;
+                if (j > 0) ptx::mbar_wait(pv_done, par ^ 1);   // P buffer and O accumulator are free again
 #pragma unroll 1
-                    for (int c = 0; c < BKV / 32; ++c) {
+                for (int c = 0; c < BKV / 32; ++c) {
+                    if (c > 0) {
                         ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
                         tmem_ld_wait_regs(va);
-                        if constexpr (BIAS) {
-#pragma unroll
-                            for (int i = 0; i < 32; ++i)
-                                if (full || (c * 32 + i >= klo && c * 32 + i < khi))
-                                    mx = fmaxf(mx, fmaf(__uint_as_float(va[i]), scale_log2e,
-                                                        rel_bias(sB, dk + c * 32 + i)));
-                        } else if (full) {
-#pragma unroll
-                            for (int i = 0; i < 32; ++i) mx = fmaxf(mx, __uint_as_float(va[i]));
-                        } else {
-#pragma unroll
-                            for (int i = 0; i < 32; ++i)
-                                if (c * 32 + i >= klo && c * 32 + i < khi) mx = fmaxf(mx, __uint_as_float(va[i]));
-                        }
                     }
-                    const float bmax = BIAS ? mx : mx * scale_log2e;   // scale > 0: max commutes with the scaling
-                    const bool move = j == 0 || bmax > m_run + 8.0f;
-                    if (move) m_new = fmaxf(m_run, bmax);
-                    const float m_safe = m_new == -INFINITY ? 0.f : m_new;
-                    if (move) alpha = ex2(m_run - m_safe);   // 0 on the first block
-                    if (j > 0) ptx::mbar_wait(pv_done, par ^ 1);   // P buffer and O accumulator are free again
+                    if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r, sB, dk);
+                    else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r, sB, dk);
+                }
+                m_new = m_ref;
+                const float m_true = fmaxf(m_ref, BIAS ? mx : mx * scale_log2e);
+                const bool exceeded = m_true > m_safe + 8.0f;
+                if (__any_sync(0xffffffffu, exceeded)) {
+                    // exact update for this block: reference = true running maximum, P recomputed
+                    m_new = m_true;
+                    const float ms2 = m_new == -INFINITY ? 0.f : m_new;
+                    alpha = ex2(m_run - ms2);   // 0 on the first block; 1 for rows whose reference did not move
+                    lsum = 0.f;
                     float dummy = -INFINITY;
 #pragma unroll 1
                     for (int c = 0; c < BKV / 32; ++c) {
                         ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
                         tmem_ld_wait_regs(va);
-                        if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, dummy, sP, r, sB, dk);
-                        else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, dummy, sP, r, sB, dk);
-                    }
-                } else {
-                    // ---- one pass: reference = running reference (first block: max of the row's first 32 scores);
-                    //      the exact maximum is tracked on the side and only checked afterwards
-                    ptx::tmem_ld_32x32b_x32(lane_addr + S_COL, va);
-                    tmem_ld_wait_regs(va);
-                    float m_ref = m_run;
-                    if (j == 0) {
-                        float c0 = -INFINITY;
-                        if constexpr (BIAS) {
-#pragma unroll
-                            for (int i = 0; i < 32; ++i)
-                                if (full || (i >= klo && i < khi))
-                                    c0 = fmaxf(c0, fmaf(__uint_as_float(va[i]), scale_log2e, rel_bias(sB, dk + i)));
-                            m_ref = c0;
-                        } else {
-#pragma unroll
-                            for (int i = 0; i < 32; ++i)
-                                if (full || (i >= klo && i < khi)) c0 = fmaxf(c0, __uint_as_float(va[i]));
-                            m_ref = c0 * scale_log2e;
-                        }
-                    }
-                    const float m_safe = m_ref == -INFINITY ? 0.f : m_ref;
-                    if (j > 0) ptx::mbar_wait(pv_done, par ^ 1);
-                    if (SM == 2) {
-                        // 16-column half chunks through two 16-register buffers inside ONE loop body: the next half's
-                        // tcgen05.ld is in flight while this half is exponentiated (same code size and registers as the
-                        // 32-column version; the round-2 attempt with two 32-register buffers and an unrolled body lost
-                        // more to instruction fetch than it hid)
-                        uint32_t vb[16], vlo[16];
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) vlo[i] = va[i];   // columns 0-15 are already here (reference pass)
-                        float ls4[4] = {0.f, 0.f, 0.f, 0.f}, mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-#pragma unroll 1
-                        for (int c = 0; c < BKV / 32; ++c) {
-                            if (c > 0) tmem_ld_wait_regs16(vlo);
-                            ptx::tmem_ld_32x32b_x16(lane_addr + S_COL + c * 32 + 16, vb);
-                            if (full)
-                                softmax_half_chunk<true, BIAS>(vlo, c * 32, klo, khi, scale_log2e, m_safe, ls4, mx4, sP, r,
-                                                               sB, dk);
-                            else
-                                softmax_half_chunk<false, BIAS>(vlo, c * 32, klo, khi, scale_log2e, m_safe, ls4, mx4, sP,
-                                                                r, sB, dk);
-                            tmem_ld_wait_regs16(vb);
-                            if (c + 1 < BKV / 32) ptx::tmem_ld_32x32b_x16(lane_addr + S_COL + (c + 1) * 32, vlo);
-                            if (full)
-                                softmax_half_chunk<true, BIAS>(vb, c * 32 + 16, klo, khi, scale_log2e, m_safe, ls4, mx4,
-                                                               sP, r, sB, dk);
-                            else
-                                softmax_half_chunk<false, BIAS>(vb, c * 32 + 16, klo, khi, scale_log2e, m_safe, ls4, mx4,
-                                                                sP, r, sB, dk);
-                        }
-                        lsum = (ls4[0] + ls4[1]) + (ls4[2] + ls4[3]);
-                        mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-                    } else {         // SM == 1: one buffer, one loop body
-#pragma unroll 1
-                        for (int c = 0; c < BKV / 32; ++c) {
-                            if (c > 0) {
-                                ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
-                                tmem_ld_wait_regs(va);
-                            }
-                            if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r, sB, dk);
-                            else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, m_safe, lsum, mx, sP, r, sB, dk);
-                        }
-                    }
-                    m_new = m_ref;
-                    const float m_true = fmaxf(m_ref, BIAS ? mx : mx * scale_log2e);
-                    const bool exceeded = m_true > m_safe + 8.0f;
-                    if (__any_sync(0xffffffffu, exceeded)) {
-                        // exact update for this block: reference = true running maximum, P recomputed
-                        m_new = m_true;
-                        const float ms2 = m_new == -INFINITY ? 0.f : m_new;
-                        alpha = ex2(m_run - ms2);   // 0 on the first block; 1 for rows whose reference did not move
-                        lsum = 0.f;
-                        float dummy = -INFINITY;
-#pragma unroll 1
-                        for (int c = 0; c < BKV / 32; ++c) {
-                            ptx::tmem_ld_32x32b_x32(lane_addr + S_COL + c * 32, va);
-                            tmem_ld_wait_regs(va);
-                            if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r, sB, dk);
-                            else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r, sB, dk);
-                        }
+                        if (full) softmax_chunk<true, BIAS>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r, sB, dk);
+                        else softmax_chunk<false, BIAS>(va, c, klo, khi, scale_log2e, ms2, lsum, dummy, sP, r, sB, dk);
                     }
                 }
                 if (j == 0) alpha = 0.f;   // nothing accumulated yet (l_run == 0, O is overwritten by the first PV)
@@ -916,39 +791,14 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap, const __nv_bfloat1
 using KernelFn = void (*)(const CUtensorMap, const __nv_bfloat16*, __nv_bfloat16*, int, int, int, const int32_t*, float,
                           int, int, int, int, int, int, const float*);
 
-template <int SM>
-static KernelFn kernel_for(int mask, bool packed) {
-    static const KernelFn table[2][3] = {
-        {tc::attention_tc_kernel<MASK_NONE, false, SM, false>, tc::attention_tc_kernel<MASK_CAUSAL, false, SM, false>,
-         tc::attention_tc_kernel<MASK_KEYLEN, false, SM, false>},
-        {tc::attention_tc_kernel<MASK_NONE, true, SM, false>, tc::attention_tc_kernel<MASK_CAUSAL, true, SM, false>,
-         tc::attention_tc_kernel<MASK_KEYLEN, true, SM, false>}};
-    return table[packed ? 1 : 0][mask];
-}
-
-// relative-position bias variants: MASK_NONE and MASK_KEYLEN (no model combines the bias with causal masking)
-template <int SM>
-static KernelFn bias_kernel_for(int mask, bool packed) {
-    static const KernelFn table[2][2] = {
-        {tc::attention_tc_kernel<MASK_NONE, false, SM, true>, tc::attention_tc_kernel<MASK_KEYLEN, false, SM, true>},
-        {tc::attention_tc_kernel<MASK_NONE, true, SM, true>, tc::attention_tc_kernel<MASK_KEYLEN, true, SM, true>}};
-    return table[packed ? 1 : 0][mask == MASK_KEYLEN ? 1 : 0];
-}
-
-static KernelFn pick_kernel(int sm, int mask, bool packed, bool bias = false) {
-    if (bias) {
-        switch (sm) {
-            case 0: return bias_kernel_for<0>(mask, packed);
-            case 2: return bias_kernel_for<2>(mask, packed);
-            default: return bias_kernel_for<1>(mask, packed);
-        }
-    }
-    switch (sm) {
-        case 0: return kernel_for<0>(mask, packed);
-        case 2: return kernel_for<2>(mask, packed);
-        default: return kernel_for<1>(mask, packed);
-    }
-}
+// [bias][packed][mask]; no model combines the relative-position bias with causal masking (launch_tc rejects it)
+static const KernelFn kernels[2][2][3] = {
+    {{tc::attention_tc_kernel<MASK_NONE, false, false>, tc::attention_tc_kernel<MASK_CAUSAL, false, false>,
+      tc::attention_tc_kernel<MASK_KEYLEN, false, false>},
+     {tc::attention_tc_kernel<MASK_NONE, true, false>, tc::attention_tc_kernel<MASK_CAUSAL, true, false>,
+      tc::attention_tc_kernel<MASK_KEYLEN, true, false>}},
+    {{tc::attention_tc_kernel<MASK_NONE, false, true>, nullptr, tc::attention_tc_kernel<MASK_KEYLEN, false, true>},
+     {tc::attention_tc_kernel<MASK_NONE, true, true>, nullptr, tc::attention_tc_kernel<MASK_KEYLEN, true, true>}}};
 
 int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W, int H, int mask, const int32_t* kv_len,
               const float* bias_log2, cudaStream_t stream) {
@@ -960,29 +810,15 @@ int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W,
     if (bias && mask == MASK_CAUSAL)
         fail(B200_ERR_INTERNAL, "attention: causal masking takes no relative-position bias");
     const uint32_t smem = bias ? tc::SMEM_BYTES_BIAS : tc::SMEM_BYTES;
-    // softmax schedule (see the kernel's SM parameter); MARQO_B200_ATTN_SOFTMAX=0|1|2 overrides for A/B timing
-    static const int softmax_mode = [] {
-        const char* e = getenv("MARQO_B200_ATTN_SOFTMAX");
-        return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : tc::DEFAULT_SOFTMAX_MODE;
-    }();
     static std::once_flag once;
     std::call_once(once, [] {
-        for (int sm = 0; sm < 3; ++sm)
+        for (int bs = 0; bs < 2; ++bs)
             for (int pk = 0; pk < 2; ++pk)
                 for (int mk = 0; mk < 3; ++mk)
-                    MB_CUDA(cudaFuncSetAttribute(pick_kernel(sm, mk, pk != 0), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                 (int)tc::SMEM_BYTES));
+                    if (kernels[bs][pk][mk])
+                        MB_CUDA(cudaFuncSetAttribute(kernels[bs][pk][mk], cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                     (int)(bs ? tc::SMEM_BYTES_BIAS : tc::SMEM_BYTES)));
     });
-    static std::once_flag once_bias;
-    if (bias)
-        std::call_once(once_bias, [] {
-            for (int sm = 0; sm < 3; ++sm)
-                for (int pk = 0; pk < 2; ++pk)
-                    for (int mk : {(int)MASK_NONE, (int)MASK_KEYLEN})
-                        MB_CUDA(cudaFuncSetAttribute(pick_kernel(sm, mk, pk != 0, true),
-                                                     cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                     (int)tc::SMEM_BYTES_BIAS));
-        });
     // one tensor map over the packed [B*S, 3W] matrix serves Q, K and V tiles (64 columns x 128 rows, 128B swizzle);
     // rows past the end of the matrix are zero-filled, rows of the next sequence are masked by key index
     CUtensorMap tmap = make_tmap_2d(qkv, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, (uint64_t)3 * W, (uint64_t)B * S,
@@ -997,7 +833,7 @@ int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W,
         const int groups = (B + pack - 1) / pack;
         const int total_items = groups * H;
         const int grid = std::min(2 * sm_count(device), total_items);
-        pick_kernel(softmax_mode, mask, true, bias)<<<grid, tc::THREADS, smem, stream>>>(
+        kernels[bias][1][mask]<<<grid, tc::THREADS, smem, stream>>>(
             tmap, qkv, out, S, W, H, kv_len, scale_log2e, /*s_main=*/1 << 30, 0, /*q_blocks=*/1, total_items, pack, B,
             bias_log2);
         MB_CUDA(cudaGetLastError());
@@ -1017,7 +853,7 @@ int launch_tc(const __nv_bfloat16* qkv, __nv_bfloat16* out, int B, int S, int W,
     int grid = 2 * sm_count(device);
     if ((q_blocks & 1) == 0 && (grid & 1) == 0) grid -= 1;
     grid = std::min(grid, total_items);
-    pick_kernel(softmax_mode, mask, false, bias)<<<grid, tc::THREADS, smem, stream>>>(
+    kernels[bias][0][mask]<<<grid, tc::THREADS, smem, stream>>>(
         tmap, qkv, out, S, W, H, kv_len, scale_log2e, s_main, inline_rows, q_blocks, total_items, 1, B, bias_log2);
     MB_CUDA(cudaGetLastError());
     return 1;

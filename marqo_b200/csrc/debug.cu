@@ -116,53 +116,6 @@ int b200_debug_patch_embed(int device, const uint8_t* hwc, int n, int S, int pat
     });
 }
 
-int b200_debug_gemm_ln(int device, const float* A, const float* W, const float* bias, const float* residual, int M, int N,
-                       int K, const float* gamma, const float* beta, float eps, int in_place, int repeats, float* out_x,
-                       float* out_ln) {
-    return guarded([&] {
-        MB_CHECK_ARG(A && W && gamma && beta && out_x && out_ln, "NULL buffer");
-        MB_CHECK_ARG(M > 0 && N > 0 && K > 0 && repeats > 0, "M, N, K, repeats must be positive");
-        require_device(device);
-        DeviceGuard g(device);
-        Scratch sc;
-        MB_CUDA(cudaStreamCreate(&sc.s));
-        __nv_bfloat16* dA = sc.upload_bf16(A, (size_t)M * K);
-        __nv_bfloat16* dW = sc.upload_bf16(W, (size_t)N * K);
-        float* dOut = sc.alloc<float>((size_t)M * N);
-        __nv_bfloat16* dLnB = sc.alloc<__nv_bfloat16>((size_t)M * N);
-        float* dLnF = sc.alloc<float>((size_t)M * N);
-        const size_t strips = (size_t)M / 32 + 2;
-        int* dCnt = sc.alloc<int>(2 * strips);   // two arrays: each launch counts in one and zeroes the other
-        MB_CUDA(cudaMemsetAsync(dCnt, 0, 2 * strips * 4, sc.s));
-        float2* dStats = sc.alloc<float2>((size_t)M * gemm::LN_MAX_PARTS);
-        gemm::Epilogue ep;
-        ep.bias = bias ? sc.upload(bias, (size_t)N) : nullptr;
-        ep.residual = residual ? sc.upload(residual, (size_t)M * N) : nullptr;
-        ep.ldr = N;
-        ep.ldo = N;
-        ep.out = dOut;
-        ep.out_fp32 = 1;
-        ep.ln_gamma = sc.upload(gamma, (size_t)N);
-        ep.ln_beta = sc.upload(beta, (size_t)N);
-        ep.ln_eps = eps;
-        ep.ln_out_bf16 = dLnB;
-        ep.ln_out_f32 = in_place ? dOut : nullptr;   // BERT post-LN: the normalised rows replace the fp32 output
-        ep.ln_stats = dStats;
-        // repeated launches alternate between the two counter arrays, as out_proj / fc2 do in the model
-        for (int i = 0; i < repeats; ++i) {
-            ep.ln_counters = dCnt + (i & 1) * strips;
-            ep.ln_zero = dCnt + ((i + 1) & 1) * strips;
-            gemm::launch(dA, K, dW, M, N, K, ep, sm_count(device), sc.s);
-        }
-        const long long n = (long long)M * N;
-        bf16_to_f32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, sc.s>>>(dLnB, dLnF, n);
-        MB_CUDA(cudaGetLastError());
-        MB_CUDA(cudaMemcpyAsync(out_x, dOut, (size_t)M * N * 4, cudaMemcpyDeviceToHost, sc.s));
-        MB_CUDA(cudaMemcpyAsync(out_ln, dLnF, (size_t)M * N * 4, cudaMemcpyDeviceToHost, sc.s));
-        MB_CUDA(cudaStreamSynchronize(sc.s));
-    });
-}
-
 int b200_debug_gemm(int device, const float* A, const float* W, const float* bias, const float* residual, int M, int N,
                     int K, int act, int out_bf16, int in_place, float* out) {
     return guarded([&] {

@@ -1,6 +1,5 @@
 #include "gemm.cuh"
 
-#include <cstdlib>
 #include <mutex>
 
 #include "ptx.cuh"
@@ -158,101 +157,6 @@ __device__ __forceinline__ void sts_f4(uint32_t a, float x, float y, float z, fl
 }
 __device__ __forceinline__ void sts_u4(uint32_t a, uint32_t x, uint32_t y, uint32_t z, uint32_t w) {
     asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(a), "r"(x), "r"(y), "r"(z), "r"(w) : "memory");
-}
-
-// ---- fused LayerNorm (gemm.cuh: Epilogue::ln_*) ----
-// Chan et al.: merge (n_a, mean_a, M2_a) with (n_b, mean_b, M2_b)
-__device__ __forceinline__ void chan_merge(float& n_a, float& mean_a, float& m2_a, float n_b, float mean_b, float m2_b) {
-    const float n = n_a + n_b;
-    const float delta = mean_b - mean_a;
-    const float w = n_b / n;
-    mean_a = fmaf(delta, w, mean_a);
-    m2_a = m2_a + m2_b + delta * delta * n_a * w;
-    n_a = n;
-}
-
-// Normalise the 32 x (32 * CHUNKS) sub-tile at (row0, col0) that THIS warp wrote one tile ago (same lane -> address mapping
-// as the flush, so its own stores are visible to it), once all column parts of the strip have published their statistics.
-template <int CHUNKS>
-__device__ __forceinline__ void ln_apply_subtile(const Epilogue& ep, int M, int N, int row0, int col0, int nparts, int lane) {
-    const int srow = lane >> 3, sunit = lane & 7;
-    const int* cnt = ep.ln_counters + (row0 >> 5);
-    if (lane == 0) {
-        int seen;
-        uint64_t t0 = 0;
-        uint32_t spins = 0;
-        while (true) {
-            asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(seen) : "l"(cnt) : "memory");
-            if (seen >= nparts) break;
-            if (t0 == 0) t0 = ptx::globaltimer_ns();
-            if ((++spins & 0xff) == 0 && ptx::globaltimer_ns() - t0 > 2000000000ull) {
-                printf("marqo_b200: fused LayerNorm strip %d never completed (%d of %d parts)\n", row0 >> 5, seen, nparts);
-                __trap();
-            }
-        }
-    }
-    __syncwarp();
-    if (ep.ln_debug_skip) return;
-    // lane == row: merge the strip's partial statistics
-    float mean = 0.f, rstd = 0.f;
-    {
-        const int row = row0 + lane;
-        if (row < M) {
-            const float2* st = ep.ln_stats + (size_t)row * LN_MAX_PARTS;
-            const float pn = (float)(N / nparts);
-            float2 sv[LN_MAX_PARTS];   // all parts in flight at once (one L2 round trip), then the merge chain
-#pragma unroll
-            for (int k = 0; k < LN_MAX_PARTS; ++k)
-                if (k < nparts) sv[k] = __ldcg(st + k);
-            float n = pn, m2 = sv[0].y;
-            mean = sv[0].x;
-#pragma unroll
-            for (int k = 1; k < LN_MAX_PARTS; ++k)
-                if (k < nparts) chan_merge(n, mean, m2, pn, sv[k].x, sv[k].y);
-            rstd = 1.0f / sqrtf(m2 / (float)N + ep.ln_eps);
-        }
-    }
-    const float* xo = reinterpret_cast<const float*>(ep.out);
-    // two 32-column chunks per step: 16 independent 16-byte loads in flight per lane (the epilogue has only 8 warps per SM,
-    // so memory-level parallelism has to come from each of them)
-    constexpr int STEP = CHUNKS >= 2 ? 2 : 1;
-#pragma unroll 1
-    for (int c = 0; c < CHUNKS; c += STEP) {
-        float4 x[STEP][8];
-#pragma unroll
-        for (int cc = 0; cc < STEP; ++cc) {
-            const int col = col0 + (c + cc) * 32 + sunit * 4;
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int row = row0 + i * 4 + srow;
-                x[cc][i] = row < M ? __ldcg(reinterpret_cast<const float4*>(xo + (size_t)row * N + col))
-                                   : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-        }
-#pragma unroll
-        for (int cc = 0; cc < STEP; ++cc) {
-            const int col = col0 + (c + cc) * 32 + sunit * 4;
-            const float4 g = __ldg(reinterpret_cast<const float4*>(ep.ln_gamma + col));
-            const float4 b = __ldg(reinterpret_cast<const float4*>(ep.ln_beta + col));
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int rr = i * 4 + srow;
-                const float mu = __shfl_sync(0xffffffffu, mean, rr), rs = __shfl_sync(0xffffffffu, rstd, rr);
-                const int row = row0 + rr;
-                if (row < M) {
-                    float4 y;
-                    y.x = (x[cc][i].x - mu) * rs * g.x + b.x;
-                    y.y = (x[cc][i].y - mu) * rs * g.y + b.y;
-                    y.z = (x[cc][i].z - mu) * rs * g.z + b.z;
-                    y.w = (x[cc][i].w - mu) * rs * g.w + b.w;
-                    if (ep.ln_out_f32) *reinterpret_cast<float4*>(ep.ln_out_f32 + (size_t)row * N + col) = y;
-                    if (ep.ln_out_bf16)
-                        *reinterpret_cast<uint2*>(ep.ln_out_bf16 + (size_t)row * N + col) =
-                            make_uint2(pack_bf16x2(y.x, y.y), pack_bf16x2(y.z, y.w));
-                }
-            }
-        }
-    }
 }
 
 template <int BN, int EW, bool GATHER>
@@ -425,7 +329,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                     // the compiler if-converted the switch and every element paid for erf-GELU AND QuickGELU (two ex2 and
                     // a reciprocal, ~40 instructions per element in the r02 SASS; fc1 was epilogue-bound at 73 % tensor pipe)
                     uint32_t pk[16];
-                    if (ep.act == ACT_GELU && !ep.act_fp32) {
+                    if (ep.act == ACT_GELU) {
                         // packed-half erf-GELU: two elements per instruction
 #pragma unroll
                         for (int j = 0; j < 16; ++j) {
@@ -433,10 +337,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                             pk[j] = pack_bf16x2(y.x, y.y);
                         }
                     } else {
-                        if (ep.act == ACT_GELU) {
-#pragma unroll
-                            for (int j = 0; j < 32; ++j) f[j] = gelu_erf(f[j]);
-                        } else if (ep.act == ACT_QUICKGELU) {
+                        if (ep.act == ACT_QUICKGELU) {
 #pragma unroll
                             for (int j = 0; j < 32; ++j) f[j] = quick_gelu(f[j]);
                         }
@@ -483,8 +384,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
         uint8_t* res_buf = stage_buf + 32 * 128 + (GATHER ? 128 : 0);   // residual block of the chunk about to be processed
         // fp32 results without token remap leave through TMA (one bulk tensor store per 32 x 32 block instead of 8 shared
         // loads + 8 global stores + their address arithmetic per lane), residual blocks arrive through TMA: p.tma_io.
-        // (Not with the fused LayerNorm: its strip counters must not run ahead of asynchronous stores.)
-        const bool tma_io = !GATHER && p.tma_io != 0 && ep.ln_gamma == nullptr;
+        const bool tma_io = !GATHER && p.tma_io != 0;
         uint64_t* my_res_full = &res_full[warp - 2];
         uint32_t res_phase = 0;
         const int esz = ep.out_fp32 ? 4 : 2;                  // output element size
@@ -493,9 +393,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
         // residual GEMMs (fp32 out in this engine) flush after every chunk
         const int chunks_per_flush = (ep.out_fp32 || residual) ? 1 : cols_per_flush / 32;
         const int srow = lane >> 3, sunit = lane & 7;         // coalesced phase: 4 rows x 8 sixteen-byte units per instr
-        const bool ln_on = !GATHER && ep.ln_gamma != nullptr;
-        const int ln_parts = p.N / HALF_COLS;                 // column parts (= statistics writers) per row
-        int pend_row0 = -1, pend_col0 = 0;                    // fused LayerNorm: the sub-tile still to be normalised
         // Residual blocks travel global -> shared memory asynchronously, one chunk AHEAD of their use (and across the
         // tile boundary: the next tile's first block is requested before this warp waits for that accumulator), in the
         // swizzled layout the lane == row read expects.  The r02 profile had out_proj (K = 1024: a tile every ~7 us) at
@@ -542,7 +439,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
             const int m0 = ((t / p.tiles_n) * CLUSTER + (int)crank) * BM;
             const int nt0 = (t % p.tiles_n) * BN + half * HALF_COLS;
             const int wrow0 = m0 + sp * 32;                   // first row of this warp's 32-row band
-            float st_n = 0.f, st_mean = 0.f, st_m2 = 0.f;     // fused LayerNorm: this lane's row over this warp's columns
             // (not for long K: a tile of fc2, K = 4096, takes ~28 us during which ~80 MB stream through the L2 — the lines
             // were evicted again before their use and the residual was fetched from HBM twice: r01/r02 ncu 1.32 GB per
             // launch against 1.085 GB algorithmic.  Its epilogue has four times the slack to take the HBM latency itself.)
@@ -655,22 +551,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                         if (c + 1 < CHUNKS) prefetch_residual(t, c + 1);
                         else prefetch_residual(t + num_clusters, 0);
                     }
-                    if (ln_on) {   // (mean, M2) of this chunk's 32 values of the lane's row, merged into the running pair
-                        float cs = 0.f;
-#pragma unroll
-                        for (int j = 0; j < 32; ++j) cs += f[j];
-                        const float cm = cs * (1.0f / 32.0f);
-                        float cq = 0.f;
-#pragma unroll
-                        for (int j = 0; j < 32; ++j) cq = fmaf(f[j] - cm, f[j] - cm, cq);
-                        if (st_n == 0.f) {
-                            st_n = 32.f;
-                            st_mean = cm;
-                            st_m2 = cq;
-                        } else {
-                            chan_merge(st_n, st_mean, st_m2, 32.f, cm, cq);
-                        }
-                    }
                     // (2) own row -> staging buffer (swizzled 16-byte units)
                     if (tma_io) {   // the previous block's bulk store must have read the buffer out
                         if (lane == 0) ptx::tma_store_wait_read<0>();
@@ -717,33 +597,11 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ 
                     __syncwarp();
                 }
             }
-            if (!GATHER && ln_on) {
-                const bool contributes = has_cols && nt0 < p.N && wrow0 < p.M;
-                if (contributes) {
-                    // publish this warp's per-row statistics, then count the strip's writers.  One release atomic per warp
-                    // covers the whole warp's stores (they are ordered before it by the warp barrier).  NOT
-                    // __threadfence(): that is fence.sc.gpu.
-                    const int row = wrow0 + lane;
-                    if (row < p.M) ep.ln_stats[(size_t)row * LN_MAX_PARTS + nt0 / HALF_COLS] = make_float2(st_mean, st_m2);
-                    __syncwarp();
-                    if (lane == 0)
-                        asm volatile("red.release.gpu.global.add.s32 [%0], 1;" ::"l"(ep.ln_counters + (wrow0 >> 5)) : "memory");
-                }
-                // the sub-tile written one tile ago: its strip has had a whole tile's time to complete.  (Doing this before
-                // the wait for the next accumulator instead — "in the idle time" — measured slower: 46.5 vs 44.5 ms per step
-                // with fc2 fused, because it delays the epilogue whenever the accumulator is already there.)
-                if (pend_row0 >= 0) ln_apply_subtile<CHUNKS>(ep, p.M, p.N, pend_row0, pend_col0, ln_parts, lane);
-                pend_row0 = contributes ? wrow0 : -1;
-                pend_col0 = nt0;
-            }
-            if (!GATHER && ep.ln_zero != nullptr && half == 0 && nt0 == 0 && lane == 0 && wrow0 < p.M)
-                ep.ln_zero[wrow0 >> 5] = 0;   // the other counter array: ready for the next fused GEMM
             if (++acc == ACC_STAGES) {
                 acc = 0;
                 acc_phase ^= 1;
             }
         }
-        if (!GATHER && ln_on && pend_row0 >= 0) ln_apply_subtile<CHUNKS>(ep, p.M, p.N, pend_row0, pend_col0, ln_parts, lane);
         if (tma_io && lane == 0) ptx::tma_store_wait<0>();
     } else if (GATHER && warp >= 2 + EW) {
         // ---------------------------------------------------------------- patch gather (uint8 HWC -> bf16 A stage)
@@ -902,8 +760,7 @@ static void launch_bn(const __nv_bfloat16* A, int lda, const __nv_bfloat16* W, i
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     // fp32 output without token remap: the epilogue's 32 x 32 blocks (128-byte rows, 128B swizzle) go through TMA
-    static const bool no_tma_io = getenv("MARQO_B200_GEMM_NO_TMA_EPILOGUE") != nullptr;   // A/B timing switch
-    p.tma_io = (!GATHER && EW == 8 && !no_tma_io && ep.out_fp32 && ep.remap_group == 0 && ep.rowbias == nullptr &&
+    p.tma_io = (!GATHER && EW == 8 && ep.out_fp32 && ep.remap_group == 0 && ep.rowbias == nullptr &&
                 ep.ldo % 4 == 0 && (ep.residual == nullptr || ep.ldr % 4 == 0) &&
                 (reinterpret_cast<uintptr_t>(ep.out) & 15) == 0 && (reinterpret_cast<uintptr_t>(ep.residual) & 15) == 0)
                    ? 1 : 0;
@@ -952,19 +809,9 @@ void launch(const __nv_bfloat16* A, int lda, const __nv_bfloat16* W, int M, int 
         const long long out_rows = (long long)M + (ep.remap_group > 0 ? M / ep.remap_group + 1 : 0) + 256;
         if (out_rows * ep.ldo >= (1LL << 32)) fail(B200_ERR_UNSUPPORTED, "gemm: output of %lld x %d elements is too large", out_rows, ep.ldo);
     }
-    if (ep.ln_gamma != nullptr) {
-        if (!ep.out_fp32 || ep.ldo != N || N % 128 != 0 || N > 1024 || ep.remap_group != 0 || !ep.ln_beta ||
-            !ep.ln_counters || !ep.ln_stats || (!ep.ln_out_bf16 && !ep.ln_out_f32))
-            fail(B200_ERR_INTERNAL, "gemm: fused LayerNorm needs a compact fp32 output of width N %% 128 == 0, N <= 1024");
-    }
     configure();
-    // bf16 output, no residual / token scatter (QKV, fc1): the 16-warp epilogue.  MARQO_B200_GEMM_EPI8=1 keeps the
-    // general 8-warp epilogue for A/B timing.
-    static const bool force8 = [] {
-        const char* e = getenv("MARQO_B200_GEMM_EPI8");
-        return e != nullptr && e[0] == '1';
-    }();
-    const bool fast = !force8 && !ep.out_fp32 && ep.residual == nullptr && ep.rowbias == nullptr && ep.remap_group == 0;
+    // bf16 output, no residual / token scatter (QKV, fc1): the 16-warp epilogue
+    const bool fast = !ep.out_fp32 && ep.residual == nullptr && ep.rowbias == nullptr && ep.remap_group == 0;
     // Largest tile that wastes no columns, otherwise the widest one.
     if (N % 256 == 0 || N > 512) {
         if (fast) launch_bn<256, 16>(A, lda, W, M, N, K, ep, sms, stream);

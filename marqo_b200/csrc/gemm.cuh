@@ -9,14 +9,12 @@ namespace mb {
 namespace gemm {
 
 enum Act { ACT_NONE = 0, ACT_GELU = 1, ACT_QUICKGELU = 2 };
-constexpr int LN_MAX_PARTS = 16;   // column parts per row in Epilogue::ln_stats (N <= 1024, >= 64 columns per part)
 
 struct Epilogue {
     const float* bias = nullptr;      // [N]
     const float* residual = nullptr;  // fp32 [M, ldr], added after the activation
     int ldr = 0;
     int act = ACT_NONE;
-    int act_fp32 = 0;     // 1: evaluate erf-GELU in fp32 even for a bf16 output (default: packed fp16, see gemm.cu gelu_erf_h2)
     void* out = nullptr;  // bf16 or fp32 [*, ldo]
     int ldo = 0;
     int out_fp32 = 0;
@@ -24,27 +22,6 @@ struct Epilogue {
     // row b * (G + 1) + 1 + i and gets rowbias[(1 + i), :] (the positional embedding) added.
     int remap_group = 0;
     const float* rowbias = nullptr;  // fp32 [G + 1, N]
-    // Fused LayerNorm of the fp32 output rows (the residual GEMMs out_proj / fc2; replaces a separate LayerNorm launch
-    // and its HBM read of the residual stream).  Every epilogue warp owns a 32-row x HALF_COLS sub-tile of the output:
-    // while it adds bias + residual it also reduces each row's (mean, M2) over its columns (lane == row in the TMEM
-    // layout, so this is thread-local), publishes them in ln_stats and bumps the 32-row strip's counter.  One tile LATER —
-    // by then the other N tiles of that row band have normally been written too, so the wait is a formality — it merges
-    // the strip's partial statistics (Chan's formula), reads its OWN sub-tile back (L2 hits) and writes
-    // LayerNorm(row) * gamma + beta as bf16 (the next GEMM's A operand) and / or fp32 (may alias `out`: BERT's post-LN
-    // rewrites the residual stream in place).  The work is spread evenly over all epilogue warps.  (The first version
-    // let the LAST writer of a strip normalise all of it: that concentrates the work on the CTA pair that finishes a row
-    // band last, which then starts its next tile late and is last again — fc2 went from 0.375 to 1.175 ms.)
-    // Requirements: out_fp32, ldo == N, N % 128 == 0, N <= 1024, no token remap.
-    const float* ln_gamma = nullptr;   // [N]; NULL = no fused LayerNorm
-    const float* ln_beta = nullptr;    // [N]
-    float ln_eps = 1e-5f;
-    __nv_bfloat16* ln_out_bf16 = nullptr;   // [M, N] or NULL
-    float* ln_out_f32 = nullptr;            // [M, N] or NULL
-    float2* ln_stats = nullptr;             // [M, LN_MAX_PARTS] (mean, M2) per row and column part
-    int* ln_counters = nullptr;             // int32 [ceil(M / 32)], all zero on entry
-    int* ln_zero = nullptr;                 // int32 [ceil(M / 32)] zeroed by this launch (the counters of the NEXT fused
-                                            // GEMM: out_proj and fc2 alternate between two arrays); may be set alone
-    int ln_debug_skip = 0;                  // timing experiments only: publish / count but skip the normalisation
 };
 
 // A: bf16 [M, K] row-major with leading dimension lda (elements); W: bf16 [N, K] row-major (nn.Linear layout).

@@ -1,7 +1,6 @@
 #include "kernels.cuh"
 
 #include <cmath>
-#include <cstdlib>
 #include <mutex>
 #include <vector>
 
@@ -57,16 +56,15 @@ __device__ __forceinline__ void ln_row(float4 (&v)[LN_MAX_V4], int nv, int w, co
 
 // Rows are visited LAST FIRST (block 0 takes the highest rows): the GEMM that produced x wrote its row bands in ascending
 // order, so the rows it wrote last — the ones most likely still in the 126 MB L2 — are read first, and the bf16 rows this
-// kernel writes last are the low ones the next GEMM (ascending again) starts with.  `reverse` = 0 restores the forward order
-// (MARQO_B200_LN_FORWARD=1, A/B timing).
+// kernel writes last are the low ones the next GEMM (ascending again) starts with.
 __global__ void __launch_bounds__(256) layernorm_kernel(const float* __restrict__ x, long long in_stride,
                                                         const float* __restrict__ gamma, const float* __restrict__ beta,
                                                         float eps, int rows, int w, float* out_f32,
-                                                        __nv_bfloat16* out_bf16, int reverse) {
+                                                        __nv_bfloat16* out_bf16) {
     int row = blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (row >= rows) return;
-    if (reverse) row = rows - 1 - row;
+    row = rows - 1 - row;
     const int nv = w / 128;
     const float4* src = reinterpret_cast<const float4*>(x + (long long)row * in_stride);
     float4 v[LN_MAX_V4];
@@ -85,8 +83,7 @@ void layernorm(const float* x, long long in_stride, const float* gamma, const fl
                float* out_f32, __nv_bfloat16* out_bf16, cudaStream_t s) {
     if (rows <= 0) return;
     check_ln_width(w);
-    static const int reverse = getenv("MARQO_B200_LN_FORWARD") == nullptr ? 1 : 0;
-    layernorm_kernel<<<(rows + 7) / 8, 256, 0, s>>>(x, in_stride, gamma, beta, eps, rows, w, out_f32, out_bf16, reverse);
+    layernorm_kernel<<<(rows + 7) / 8, 256, 0, s>>>(x, in_stride, gamma, beta, eps, rows, w, out_f32, out_bf16);
     MB_CUDA(cudaGetLastError());
 }
 

@@ -74,9 +74,6 @@ struct b200_model {
     long long max_tokens = 0;
     float* x = nullptr;
     __nv_bfloat16 *h = nullptr, *qkv = nullptr, *o = nullptr, *u = nullptr, *patches = nullptr;
-    int* ln_counters = nullptr;   // two int32 arrays [ln_counter_stride] (out_proj / fc2), zero between uses (gemm.cuh)
-    long long ln_counter_stride = 0;
-    float2* ln_stats = nullptr;   // [max tokens, gemm::LN_MAX_PARTS] per-row partial (mean, M2)
     int32_t *aux = nullptr;           // [max_batch] eot index / kv_len
     float* out_dev = nullptr;         // [max_batch, embed]
     float* pooled = nullptr;          // [max_batch, width] LayerNorm-ed pooled rows (CLIP heads)
@@ -132,8 +129,6 @@ void model_free(b200_model* m) {
     cudaFree(m->o);
     cudaFree(m->u);
     cudaFree(m->patches);
-    cudaFree(m->ln_counters);
-    cudaFree(m->ln_stats);
     cudaFree(m->aux);
     cudaFree(m->out_dev);
     cudaFree(m->pooled);
@@ -291,57 +286,14 @@ void attend(b200_model* m, Counter& c, int B, int S, int w, int heads, int mask_
     c.n += attention::launch(m->qkv, m->o, B, S, w, heads, mask_mode, kv_len, bias_log2, m->stream);
 }
 
-// LayerNorm fused into the producing residual GEMM's epilogue (gemm.cuh: Epilogue::ln_*).  OFF by default: correct
-// (tests/test_kernels_gpu.py::test_gemm_fused_layernorm; the encoder parity tests pass with MARQO_B200_LN_FUSION=1 / 2),
-// and the publish + count part is free (40.2 ms per step with the normalisation skipped vs 42.1 with separate launches),
-// but re-reading the rows through the GEMM's 8 epilogue warps per SM is latency-bound where the standalone kernel runs at
-// the HBM roofline: ViT-L-14 b256, same box, 43.5-44.3 ms (separate) / 44.5 (fc2 fused) / 46.9 (both fused);
-// profiles/r02_ncu_summary.md §5-6 has the two schemes that were tried and their profiles.
-// MARQO_B200_GELU_FP32=1: evaluate fc1's erf-GELU in fp32 instead of packed fp16 (A/B timing and accuracy comparisons)
-bool gelu_fp32() {
-    static const bool on = getenv("MARQO_B200_GELU_FP32") != nullptr;
-    return on;
-}
-
-// 0 = separate launches, 1 = out_proj and fc2 fused, 2 = fc2 only (K = 4 * width: its epilogue has four times the slack)
-int ln_fusion_mode() {
-    static const int mode = [] {
-        const char* e = getenv("MARQO_B200_LN_FUSION");
-        return (e != nullptr && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 0;
-    }();
-    return mode;
-}
-
-// which: 0 = out_proj (counter array A, zeroes B), 1 = fc2 (counter array B, zeroes A).  The two residual GEMMs of a layer
-// alternate, so each launch finds its own counters zeroed by the previous one (both start zero).
-void fuse_ln(b200_model* m, gemm::Epilogue& e, int which, const float* gamma, const float* beta, float eps, float* out_f32,
-             __nv_bfloat16* out_bf16) {
-    e.ln_gamma = gamma;
-    e.ln_beta = beta;
-    e.ln_eps = eps;
-    e.ln_out_f32 = out_f32;
-    e.ln_out_bf16 = out_bf16;
-    e.ln_stats = m->ln_stats;
-    e.ln_counters = m->ln_counters + (which ? m->ln_counter_stride : 0);
-    e.ln_zero = m->ln_counters + (which ? 0 : m->ln_counter_stride);
-    static const bool skip = getenv("MARQO_B200_LN_DEBUG_SKIP") != nullptr;   // timing experiments only (wrong results)
-    e.ln_debug_skip = skip ? 1 : 0;
-}
-
 // Pre-LN residual blocks (open_clip ResidualAttentionBlock).  x (fp32) is the residual stream, h (bf16) the LayerNorm
-// output the next GEMM consumes: ln_1 of layer 0 is a launch of its own, every other LayerNorm runs inside the epilogue
-// of the GEMM that produces its input (out_proj -> ln_2, fc2 -> ln_1 of the next layer).
+// output the next GEMM consumes.
 void run_clip_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, int mask_mode) {
     const int M = B * S, w = T.d.width, mlp = T.d.mlp;
     const int act = m->desc.act == B200_ACT_QUICKGELU ? gemm::ACT_QUICKGELU : gemm::ACT_GELU;
-    const int fmode = ln_fusion_mode();
-    const bool fused = fmode != 0, fused_o = fmode == 1;
-    for (size_t li = 0; li < T.layers.size(); ++li) {
-        const LayerW& L = T.layers[li];
-        if (!fused || li == 0) {
-            kernels::layernorm(m->x, w, L.ln1_w, L.ln1_b, 1e-5f, M, w, nullptr, m->h, m->stream);
-            ++c.n;
-        }
+    for (const LayerW& L : T.layers) {
+        kernels::layernorm(m->x, w, L.ln1_w, L.ln1_b, 1e-5f, M, w, nullptr, m->h, m->stream);
+        ++c.n;
         gemm::Epilogue e1;
         e1.bias = L.b_qkv;
         e1.out = m->qkv;
@@ -355,19 +307,14 @@ void run_clip_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, i
         e2.out = m->x;
         e2.ldo = w;
         e2.out_fp32 = 1;
-        if (fused_o) fuse_ln(m, e2, 0, L.ln2_w, L.ln2_b, 1e-5f, nullptr, m->h);
-        else if (fused) e2.ln_zero = m->ln_counters + m->ln_counter_stride;   // re-arm fc2's counters
         linear(m, c, m->o, M, w, L.w_o, w, e2);
-        if (!fused_o) {
-            kernels::layernorm(m->x, w, L.ln2_w, L.ln2_b, 1e-5f, M, w, nullptr, m->h, m->stream);
-            ++c.n;
-        }
+        kernels::layernorm(m->x, w, L.ln2_w, L.ln2_b, 1e-5f, M, w, nullptr, m->h, m->stream);
+        ++c.n;
         gemm::Epilogue e3;
         e3.bias = L.b_fc;
         e3.act = act;
         e3.out = m->u;
         e3.ldo = mlp;
-        e3.act_fp32 = gelu_fp32() ? 1 : 0;
         linear(m, c, m->h, M, w, L.w_fc, mlp, e3);
         gemm::Epilogue e4;
         e4.bias = L.b_proj;
@@ -376,21 +323,15 @@ void run_clip_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, i
         e4.out = m->x;
         e4.ldo = w;
         e4.out_fp32 = 1;
-        if (fused && li + 1 < T.layers.size())
-            fuse_ln(m, e4, 1, T.layers[li + 1].ln1_w, T.layers[li + 1].ln1_b, 1e-5f, nullptr, m->h);
-        else if (fused)
-            e4.ln_zero = m->ln_counters;   // the last fc2 has no LayerNorm to fuse but still re-arms out_proj's counters
         linear(m, c, m->u, M, mlp, L.w_proj, w, e4);
     }
 }
 
 // Post-LN blocks (HF BertLayer / MPNetLayer); on entry x (fp32) and h (bf16) both hold the embedding LayerNorm output.
-// Both LayerNorms of a layer run inside the epilogue of the GEMM before them and rewrite x in place.  eps: 1e-12 for
-// BERT, 1e-5 for MPNet; T.rel_bias (MPNet) is added to every attention score.
+// Both LayerNorms of a layer follow the GEMM before them and rewrite x in place.  eps: 1e-12 for BERT, 1e-5 for MPNet;
+// T.rel_bias (MPNet) is added to every attention score.
 void run_bert_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, float eps) {
     const int M = B * S, w = T.d.width, mlp = T.d.mlp;
-    const int fmode = ln_fusion_mode();
-    const bool fused = fmode != 0, fused_o = fmode == 1;
     for (const LayerW& L : T.layers) {
         gemm::Epilogue e1;
         e1.bias = L.b_qkv;
@@ -405,19 +346,14 @@ void run_bert_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, f
         e2.out = m->x;
         e2.ldo = w;
         e2.out_fp32 = 1;
-        if (fused_o) fuse_ln(m, e2, 0, L.ln1_w, L.ln1_b, eps, m->x, m->h);
-        else if (fused) e2.ln_zero = m->ln_counters + m->ln_counter_stride;   // re-arm fc2's counters
         linear(m, c, m->o, M, w, L.w_o, w, e2);
-        if (!fused_o) {
-            kernels::layernorm(m->x, w, L.ln1_w, L.ln1_b, eps, M, w, m->x, m->h, m->stream);
-            ++c.n;
-        }
+        kernels::layernorm(m->x, w, L.ln1_w, L.ln1_b, eps, M, w, m->x, m->h, m->stream);
+        ++c.n;
         gemm::Epilogue e3;
         e3.bias = L.b_fc;
         e3.act = gemm::ACT_GELU;
         e3.out = m->u;
         e3.ldo = mlp;
-        e3.act_fp32 = gelu_fp32() ? 1 : 0;
         linear(m, c, m->h, M, w, L.w_fc, mlp, e3);
         gemm::Epilogue e4;
         e4.bias = L.b_proj;
@@ -426,12 +362,9 @@ void run_bert_blocks(b200_model* m, Counter& c, const TowerW& T, int B, int S, f
         e4.out = m->x;
         e4.ldo = w;
         e4.out_fp32 = 1;
-        if (fused) fuse_ln(m, e4, 1, L.ln2_w, L.ln2_b, eps, m->x, m->h);
         linear(m, c, m->u, M, mlp, L.w_proj, w, e4);
-        if (!fused) {
-            kernels::layernorm(m->x, w, L.ln2_w, L.ln2_b, eps, M, w, m->x, m->h, m->stream);
-            ++c.n;
-        }
+        kernels::layernorm(m->x, w, L.ln2_w, L.ln2_b, eps, M, w, m->x, m->h, m->stream);
+        ++c.n;
     }
 }
 
@@ -450,8 +383,7 @@ void forward_images_eager(b200_model* m, Counter& c, const uint8_t* u8, const fl
     e.out_fp32 = 1;
     e.remap_group = G;
     e.rowbias = T.pos;
-    static const bool no_gather = getenv("MARQO_B200_NO_PATCH_GATHER") != nullptr;   // A/B timing switch
-    if (u8 && T.conv_wg && !no_gather && (reinterpret_cast<uintptr_t>(u8) & 15) == 0) {
+    if (u8 && T.conv_wg && (reinterpret_cast<uintptr_t>(u8) & 15) == 0) {
         // uint8 pixels -> ToTensor + Normalize -> bf16 inside the GEMM's operand load: no patch matrix in HBM
         gemm::PatchGather pg;
         pg.img = u8;
@@ -819,11 +751,6 @@ int b200_model_finalize(b200_model* m) {
         dev_alloc((void**)&m->qkv, (size_t)m->max_tokens * max_w * 6);
         dev_alloc((void**)&m->o, (size_t)m->max_tokens * max_w * 2);
         dev_alloc((void**)&m->u, (size_t)m->max_tokens * max_mlp * 2);
-        m->ln_counter_stride = m->max_tokens / 32 + 2;
-        dev_alloc((void**)&m->ln_counters, (size_t)m->ln_counter_stride * 2 * 4);
-        MB_CUDA(cudaMemsetAsync(m->ln_counters, 0, (size_t)m->ln_counter_stride * 2 * 4, m->stream));
-        dev_alloc((void**)&m->ln_stats, (size_t)m->max_tokens * gemm::LN_MAX_PARTS * sizeof(float2));
-        MB_CUDA(cudaStreamSynchronize(m->stream));
         dev_alloc((void**)&m->aux, (size_t)m->desc.max_batch * 4);
         dev_alloc((void**)&m->out_dev, (size_t)m->desc.max_batch * E * 4);
         dev_alloc((void**)&m->pooled, (size_t)m->desc.max_batch * max_w * 4);

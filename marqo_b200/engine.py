@@ -503,22 +503,6 @@ def debug_gemm(A, W, bias=None, residual=None, act: int = 0, out_bf16: bool = Fa
     return out
 
 
-def debug_gemm_ln(A, W, bias, residual, gamma, beta, eps: float, in_place: bool = False, repeats: int = 1,
-                  device: int = 0):
-    """Residual GEMM with fused LayerNorm -> (x fp32 [M, N], LayerNorm(x) rounded to bf16 [M, N])."""
-    A, W = _as(A, np.float32), _as(W, np.float32)
-    M, K = A.shape
-    Nn = W.shape[0]
-    b = None if bias is None else _as(bias, np.float32)
-    r = None if residual is None else _as(residual, np.float32)
-    g, be = _as(gamma, np.float32), _as(beta, np.float32)
-    out_x = np.empty((M, Nn), np.float32)
-    out_ln = np.empty((M, Nn), np.float32)
-    N.check(N.load().b200_debug_gemm_ln(device, _ptr(A), _ptr(W), _ptr(b), _ptr(r), M, Nn, K, _ptr(g), _ptr(be),
-                                        float(eps), 1 if in_place else 0, repeats, _ptr(out_x), _ptr(out_ln)))
-    return out_x, out_ln
-
-
 def debug_patch_embed(images_u8, patch: int, conv_w, mean, std, pos=None, use_gather: bool = True,
                       device: int = 0) -> np.ndarray:
     """ViT patch embedding of uint8 HWC images [n, S, S, 3] -> token rows fp32 [n * (G + 1), N] (class rows zero)."""
